@@ -13,9 +13,8 @@ The reference has no tests or golden vectors of its own (SURVEY.md section 4), a
 depend on the versions of NumPy and OpenCV that happen to be installed
 (``backend/requirements.txt`` pins nothing).  The oracle is therefore pinned to the reference
 function *executed unmodified in the build container* (NumPy 2.3.5, OpenCV 4.13.0 with IPP):
-``tests/test_oracle_vs_reference.py`` checks bit-equality of this restatement against the
-reference on every branch, and ``oracle/make_golden.py`` stores outputs of the reference itself
-under ``tests/golden/``.
+``oracle/make_golden.py`` stores outputs of the reference itself under ``tests/golden/`` on every
+branch, and ``tests/test_oracle_golden.py`` checks bit-equality of this restatement against them.
 
 Third-party arithmetic restated here (none of it is vendored under /root/reference):
 

@@ -2,6 +2,7 @@
 outputs of the UNMODIFIED reference function (backend/app.py:174-250) made by
 oracle/make_golden.py.  This is what pins the oracle."""
 import hashlib
+import os
 import warnings
 
 import numpy as np
@@ -9,7 +10,7 @@ import pytest
 
 from oracle import d2pc_oracle as O
 from tests import cases
-from tests.conftest import assert_bits_equal
+from tests.conftest import GOLDEN_DIR, assert_bits_equal
 
 
 def _sha(a):
@@ -165,7 +166,7 @@ def test_depth_preview_oracle_matches_reference_data_urls(small_golden):
     import json
 
     import cv2
-    lut = np.load("tests/golden/plasma_lut_bgr.npy")
+    lut = np.load(os.path.join(GOLDEN_DIR, "plasma_lut_bgr.npy"))
     names = json.loads(str(small_golden.z["__preview_names__"]))
     assert len(names) >= 3
     for name in names:

@@ -2,6 +2,7 @@
 golden vectors of the unmodified reference.  Bit-exact for xyz, rgb, masks and voxel indices;
 voxel means within 1e-5 relative (float64 atomics are order-dependent)."""
 import hashlib
+import os
 import warnings
 
 import numpy as np
@@ -9,7 +10,7 @@ import pytest
 
 from oracle import d2pc_oracle as O
 from tests import cases
-from tests.conftest import assert_bits_equal
+from tests.conftest import GOLDEN_DIR, assert_bits_equal
 
 pytestmark = pytest.mark.gpu
 
@@ -405,7 +406,7 @@ def test_bounds_equal_numpy_minmax(m):
 def test_depth_preview(m, small_golden):
     """f2: colour-mapped preview bit-exact against the oracle; data URL equal to the reference's."""
     import json
-    lut = np.load("tests/golden/plasma_lut_bgr.npy")
+    lut = np.load(os.path.join(GOLDEN_DIR, "plasma_lut_bgr.npy"))
     for name in json.loads(str(small_golden.z["__preview_names__"])):
         dep = small_golden.z[f"{name}/depth"]
         inv = bool(small_golden.z[f"{name}/invert"])
