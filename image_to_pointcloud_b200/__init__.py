@@ -11,6 +11,7 @@ from .api import create_depth_preview, depth_preview_bgr, depth_to_point_cloud, 
 from .engine import DENSITY_STEP, BatchStream, EmitResult, FrameEngine, reference_intrinsics, shard_frames
 from .hostpipe import HostFramePipeline, MultiGpuPipeline
 from ._lib import D2pcConfig, D2pcError, D2pcFrameParams, load_library
+from .normals import estimate_normals
 from .pipeline import point_cloud_stage
 from .refine import refine_point_cloud, statistical_outlier_removal
 from .writers import (las_point_records, ply_vertex_records, preview_lists, preview_rows, save_las, save_ply,
@@ -22,5 +23,6 @@ __all__ = [
     "D2pcConfig", "D2pcFrameParams", "D2pcError", "load_library",
     "preview_rows", "preview_lists", "xyz_text", "save_xyz", "las_point_records", "save_las", "ply_vertex_records",
     "save_ply", "save_point_cloud", "refine_point_cloud", "statistical_outlier_removal", "point_cloud_stage",
+    "estimate_normals",
 ]
 __version__ = "0.1.0"

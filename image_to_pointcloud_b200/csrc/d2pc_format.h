@@ -8,7 +8,8 @@
 //   save_las  (app.py:343-377): LAS 1.2 point format 2, 26-byte records,
 //             X = int32(np.round((float64(x) - offset) / 0.01)), colours clip(c,0,255).astype(uint16)*256.
 //   save_ply  (app.py:329-341, Open3D binary_little_endian): double x, y, z; uchar red, green, blue
-//             = round(clamp(float32(c / 255.0), 0, 1) * 255).
+//             = round(clamp(float32(c / 255.0), 0, 1) * 255); with normals (51 bytes): double x, y, z,
+//             nx, ny, nz; uchar red, green, blue.
 #ifndef D2PC_FORMAT_H_
 #define D2PC_FORMAT_H_
 
@@ -20,6 +21,7 @@ constexpr int kXyzMaxNumber = 1 + 20 + 1 + 6;            // sign, <= 20 integer 
 constexpr int kXyzMaxLine = 3 * kXyzMaxNumber + 3 * 11 + 6;  // three coordinates, three ints, 5 spaces + '\n'
 constexpr int kLasRecordBytes = 26;
 constexpr int kPlyRecordBytes = 27;
+constexpr int kPlyNormalRecordBytes = 51;
 
 // Writes the decimal digits of n (at least one) to out, returns the count.
 D2PC_HD int put_u64(unsigned long long n, char *out) {
@@ -144,25 +146,37 @@ D2PC_HD bool las_record(const float *p, const float *c, const double off[3], dou
   return ok;
 }
 
+D2PC_HD void put_f64(uint8_t *o, double d) {
+  unsigned long long u;
+#if defined(__CUDA_ARCH__)
+  u = (unsigned long long)__double_as_longlong(d);
+#else
+  memcpy(&u, &d, 8);
+#endif
+  put_le64(o, u);
+}
+
+// Open3D's PLY colour byte: round(clamp(float32(c / 255), 0, 1) * 255)
+D2PC_HD uint8_t ply_colour(float c) {
+  const float c32 = c / 255.0f;  // colors / 255.0 stays float32 (weak Python scalar)
+  double t = (double)c32;
+  t = t < 0.0 ? 0.0 : t;
+  t = t > 1.0 ? 1.0 : t;
+  return (t == t) ? (uint8_t)(int)floor(t * 255.0 + 0.5) : (uint8_t)0;  // std::round of a value >= 0
+}
+
 // Open3D binary PLY vertex: three float64 coordinates, three uchar colours.
 D2PC_HD void ply_record(const float *p, const float *c, uint8_t *o) {
-  for (int k = 0; k < 3; ++k) {
-    const double d = (double)p[k];
-    unsigned long long u;
-#if defined(__CUDA_ARCH__)
-    u = (unsigned long long)__double_as_longlong(d);
-#else
-    memcpy(&u, &d, 8);
-#endif
-    put_le64(o + 8 * k, u);
-  }
-  for (int k = 0; k < 3; ++k) {
-    const float c32 = c[k] / 255.0f;  // colors / 255.0 stays float32 (weak Python scalar)
-    double t = (double)c32;
-    t = t < 0.0 ? 0.0 : t;
-    t = t > 1.0 ? 1.0 : t;
-    o[24 + k] = (t == t) ? (uint8_t)(int)floor(t * 255.0 + 0.5) : (uint8_t)0;  // std::round of a value >= 0
-  }
+  for (int k = 0; k < 3; ++k) put_f64(o + 8 * k, (double)p[k]);
+  for (int k = 0; k < 3; ++k) o[24 + k] = ply_colour(c[k]);
+}
+
+// Open3D binary PLY vertex of a cloud with normals, in its writer's property order: float64 x, y, z, nx, ny, nz,
+// then uchar red, green, blue.
+D2PC_HD void ply_normal_record(const float *p, const double *nrm, const float *c, uint8_t *o) {
+  for (int k = 0; k < 3; ++k) put_f64(o + 8 * k, (double)p[k]);
+  for (int k = 0; k < 3; ++k) put_f64(o + 24 + 8 * k, nrm[k]);
+  for (int k = 0; k < 3; ++k) o[48 + k] = ply_colour(c[k]);
 }
 
 // preview stride of app.py:495-500: points[::stride] with stride = max(1, n // max_preview) when

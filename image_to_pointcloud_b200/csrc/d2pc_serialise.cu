@@ -8,6 +8,7 @@
 //                  the row's offset, 16-byte coalesced copy-out)
 //   LAS 1.2 fmt 2  26-byte records, scaled int32 coordinates, 16-bit colours  -> d2pc_las_records_enqueue
 //   PLY (Open3D)   27-byte records, float64 coordinates, uchar colours        -> d2pc_ply_records_enqueue
+//                  51-byte records, + float64 normals                        -> d2pc_ply_normal_records_enqueue
 // Every entry point works on ONE frame's rows (pointers into the [batch, N, 3] outputs of emit).
 #include "d2pc_device.cuh"
 #include "d2pc_format.h"
@@ -190,6 +191,22 @@ __global__ void __launch_bounds__(kSerThreads) ser_ply_kernel(const float *xyz, 
   });
 }
 
+__global__ void __launch_bounds__(kSerThreads) ser_ply_normal_kernel(const float *xyz, const double *normals,
+                                                                     const float *rgb, const uint32_t *count,
+                                                                     uint8_t *records) {
+  ser_records<kPlyNormalRecordBytes>(count, records, [&](uint32_t i, uint8_t *o) {
+    float p[3], c[3];
+    double nv[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      p[k] = __ldg(xyz + 3 * (size_t)i + k);
+      nv[k] = __ldg(normals + 3 * (size_t)i + k);
+      c[k] = __ldg(rgb + 3 * (size_t)i + k);
+    }
+    ply_normal_record(p, nv, c, o);
+  });
+}
+
 // per-axis min / max of the rows (float(points[:, k].min()), app.py:352, 394-399) when emit's fused bounds
 // are not at hand: keys[0..2] = min, keys[3..5] = max (ordered uint32 keys)
 __global__ void ser_bounds_init_kernel(uint32_t *keys) {
@@ -320,6 +337,17 @@ extern "C" int d2pc_ply_records_enqueue(const float *d_xyz, const float *d_rgb, 
   if (!d_xyz || !d_rgb || !d_count || !d_records) return D2PC_ERR_INVALID_ARGUMENT;
   if (capacity_rows == 0 || ((uintptr_t)d_records & 15u) != 0) return D2PC_ERR_INVALID_ARGUMENT;
   ser_ply_kernel<<<ser_tiles(capacity_rows), kSerThreads, 0, (cudaStream_t)stream>>>(d_xyz, d_rgb, d_count, d_records);
+  D2PC_CHECK_LAUNCH();
+  return D2PC_OK;
+}
+
+extern "C" int d2pc_ply_normal_records_enqueue(const float *d_xyz, const double *d_normals, const float *d_rgb,
+                                               const uint32_t *d_count, uint32_t capacity_rows, uint8_t *d_records,
+                                               void *stream) {
+  if (!d_xyz || !d_normals || !d_rgb || !d_count || !d_records) return D2PC_ERR_INVALID_ARGUMENT;
+  if (capacity_rows == 0 || ((uintptr_t)d_records & 15u) != 0) return D2PC_ERR_INVALID_ARGUMENT;
+  ser_ply_normal_kernel<<<ser_tiles(capacity_rows), kSerThreads, 0, (cudaStream_t)stream>>>(d_xyz, d_normals, d_rgb,
+                                                                                            d_count, d_records);
   D2PC_CHECK_LAUNCH();
   return D2PC_OK;
 }

@@ -3,6 +3,7 @@
 
     depth_to_point_cloud (:468-476) -> refine_point_cloud (:479) -> preview decimation (:495-506)
     -> save_point_cloud (:537) -> generate_gis_metadata bounds (:393-400)
+    [-> estimate_normals, the mesh builder's first step (:271-308), with normals=True]
 
 Called as separate drop-ins, those steps move the cloud across PCIe five times (down after the stage, up
 and down around the refinement, up again for the writer).  Here the image and the depth map go up once,
@@ -23,6 +24,7 @@ from . import _lib, writers
 from ._lib import check
 from .api import _engine_for, _image_channels, _to_host, bounds_dict, check_depth_dtype
 from .engine import DENSITY_STEP
+from .normals import estimate_normals
 from .refine import statistical_outlier_removal
 
 
@@ -30,11 +32,14 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
                       depth_scale: float = 10.0, smooth: bool = False, smooth_ksize: int = 5, fov: Optional[float] = None,
                       refine: bool = True, nb_neighbors: int = 20, std_ratio: float = 2.0,
                       output_format: Optional[str] = "ply", filename: Optional[str] = None,
-                      max_preview: int = writers.MAX_PREVIEW, return_arrays: bool = True, device=None) -> dict:
+                      max_preview: int = writers.MAX_PREVIEW, return_arrays: bool = True, normals: bool = False,
+                      normals_knn: int = 30, device=None) -> dict:
     """Returns a dict with ``points`` / ``colors`` (host float32 [M,3], if ``return_arrays``), ``point_count``,
     ``preview_points`` / ``preview_colors`` (nested lists as app.py:505-506), ``bounds`` (app.py:393-400),
     and either ``filepath`` (``filename`` given: the file the reference's writer would have put into
-    outputs/<filename>.<ext>) or ``file_bytes`` (its content)."""
+    outputs/<filename>.<ext>) or ``file_bytes`` (its content).  With ``normals`` the refined rows' normals
+    (``estimate_normals(points, knn=normals_knn)``, float64 [M,3]) are computed on the device, returned as
+    ``normals`` (if ``return_arrays``) and written into a PLY file."""
     DENSITY_STEP[density]  # KeyError first, like the reference
     lib = _lib.load_library()
     img_h, img_w = image.shape[:2]
@@ -55,8 +60,11 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
             xyz, rgb, _, _ = statistical_outlier_removal(xyz, rgb, nb_neighbors, std_ratio, return_device=True)
         m = int(xyz.shape[0])
         out = {"point_count": m}
+        nrm = estimate_normals(xyz, knn=normals_knn, return_device=True) if normals else None
         if return_arrays:
             out["points"], out["colors"] = _to_host(xyz), _to_host(rgb)   # pinned D2H at PCIe speed
+            if normals:
+                out["normals"] = nrm.cpu().numpy()
         pp, pc = writers.preview_lists(xyz, rgb, max_preview)
         out["preview_points"], out["preview_colors"] = pp, pc
         if m > 0:
@@ -69,8 +77,9 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
         fmt = (output_format or "").lower()
         if fmt:
             if fmt == "ply":
-                rec = writers.ply_vertex_records(xyz, rgb)
-                head, ext = writers.PLY_HEADER.format(n=len(rec)).encode("ascii"), "ply"
+                rec = writers.ply_vertex_records(xyz, rgb, normals=nrm)
+                header = writers.PLY_HEADER if nrm is None else writers.PLY_NORMAL_HEADER
+                head, ext = header.format(n=len(rec)).encode("ascii"), "ply"
             elif fmt in ("las", "laz"):
                 rec, offsets, mm = writers.las_point_records(xyz, rgb, 0.01)
                 head, ext = writers.las_header(len(rec), 0.01, offsets, mm), "las"

@@ -4,7 +4,7 @@ with the per-point work moved to the GPU.
     preview_lists(points, colors)            app.py:495-506   strided rows -> nested lists for the JSON
     save_xyz(points, colors, filename)       app.py:379-389   ASCII "%.6f %.6f %.6f %d %d %d" lines
     save_las(points, colors, filename)       app.py:343-377   LAS 1.2, point format 2 (scale 0.01, offset = min)
-    save_ply(points, colors, filename)       app.py:329-341   Open3D binary little-endian PLY
+    save_ply(points, colors, filename)       app.py:329-341   Open3D binary little-endian PLY (normals=: with nx, ny, nz)
     save_point_cloud(points, colors, format, filename)   app.py:310-327   the dispatcher
 
 Same signatures and return values (the file path under ``outputs/``) as the reference.  ``points`` /
@@ -35,6 +35,7 @@ logger = logging.getLogger(__name__)
 
 LAS_RECORD_BYTES = 26
 PLY_RECORD_BYTES = 27
+PLY_NORMAL_RECORD_BYTES = 51
 MAX_PREVIEW = 20000  # app.py:496
 
 
@@ -191,30 +192,53 @@ def save_las(points, colors, filename: str, device=None) -> str:
 PLY_HEADER = ("ply\nformat binary_little_endian 1.0\ncomment Created by Open3D\nelement vertex {n}\n"
               "property double x\nproperty double y\nproperty double z\n"
               "property uchar red\nproperty uchar green\nproperty uchar blue\nend_header\n")
+# Open3D's writer puts the normals after z when the cloud has them
+PLY_NORMAL_HEADER = ("ply\nformat binary_little_endian 1.0\ncomment Created by Open3D\nelement vertex {n}\n"
+                     "property double x\nproperty double y\nproperty double z\n"
+                     "property double nx\nproperty double ny\nproperty double nz\n"
+                     "property uchar red\nproperty uchar green\nproperty uchar blue\nend_header\n")
 
 
-def ply_vertex_records(points, colors, device=None) -> np.ndarray:
-    """-> uint8 [n, 27]: float64 x, y, z and uchar r, g, b per vertex."""
+def _device_normals(normals, n: int, dev) -> torch.Tensor:
+    if isinstance(normals, torch.Tensor):
+        nrm = normals.to(dev)
+    else:
+        nrm = torch.from_numpy(np.ascontiguousarray(normals, dtype=np.float64)).to(dev)
+    if nrm.dtype != torch.float64 or tuple(nrm.shape) != (n, 3):
+        raise ValueError("normals must be float64 [N, 3] for N points")
+    return nrm.contiguous()
+
+
+def ply_vertex_records(points, colors, device=None, normals=None) -> np.ndarray:
+    """-> uint8 [n, 27]: float64 x, y, z and uchar r, g, b per vertex; with ``normals`` (float64 [n, 3]) uint8
+    [n, 51]: float64 x, y, z, nx, ny, nz and uchar r, g, b."""
     lib = _lib.load_library()
     xyz, rgb, count, n = _device_rows(points, colors, device)
+    rb = PLY_RECORD_BYTES if normals is None else PLY_NORMAL_RECORD_BYTES
     if n == 0:
-        return np.zeros((0, PLY_RECORD_BYTES), np.uint8)
+        return np.zeros((0, rb), np.uint8)
     dev = xyz.device
     with torch.cuda.device(dev):
-        rec = torch.empty(n * PLY_RECORD_BYTES + 16, dtype=torch.uint8, device=dev)
-        check(lib.d2pc_ply_records_enqueue(xyz.data_ptr(), rgb.data_ptr(), count.data_ptr(), n, rec.data_ptr(),
-                                           _stream(dev)), "d2pc_ply_records_enqueue")
-        host = torch.empty(n * PLY_RECORD_BYTES, dtype=torch.uint8, pin_memory=True)
-        host.copy_(rec[:n * PLY_RECORD_BYTES])
-        return host.numpy().reshape(n, PLY_RECORD_BYTES)
+        rec = torch.empty(n * rb + 16, dtype=torch.uint8, device=dev)
+        if normals is None:
+            check(lib.d2pc_ply_records_enqueue(xyz.data_ptr(), rgb.data_ptr(), count.data_ptr(), n, rec.data_ptr(),
+                                               _stream(dev)), "d2pc_ply_records_enqueue")
+        else:
+            nrm = _device_normals(normals, n, dev)
+            check(lib.d2pc_ply_normal_records_enqueue(xyz.data_ptr(), nrm.data_ptr(), rgb.data_ptr(), count.data_ptr(),
+                                                      n, rec.data_ptr(), _stream(dev)), "d2pc_ply_normal_records_enqueue")
+        host = torch.empty(n * rb, dtype=torch.uint8, pin_memory=True)
+        host.copy_(rec[:n * rb])
+        return host.numpy().reshape(n, rb)
 
 
-def save_ply(points, colors, filename: str, device=None) -> str:
-    """Save as PLY format (reference save_ply, app.py:329-341)."""
+def save_ply(points, colors, filename: str, device=None, normals=None) -> str:
+    """Save as PLY format (reference save_ply, app.py:329-341); with ``normals`` the vertices carry nx, ny, nz."""
     filepath = f"outputs/{filename}.ply"
-    rec = ply_vertex_records(points, colors, device)
+    rec = ply_vertex_records(points, colors, device, normals=normals)
+    header = PLY_HEADER if normals is None else PLY_NORMAL_HEADER
     with open(filepath, "wb") as f:
-        f.write(PLY_HEADER.format(n=len(rec)).encode("ascii"))
+        f.write(header.format(n=len(rec)).encode("ascii"))
         f.write(rec.tobytes())
     return filepath
 

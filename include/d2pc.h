@@ -265,6 +265,12 @@ int d2pc_las_records_enqueue(const float *d_xyz, const float *d_rgb, const uint3
 int d2pc_ply_records_enqueue(const float *d_xyz, const float *d_rgb, const uint32_t *d_count,
                              uint32_t capacity_rows, uint8_t *d_records, void *stream);
 
+/* The same vertices for a cloud with normals, 51 bytes each in Open3D's property order: float64 x, y, z, nx, ny, nz;
+ * uchar red, green, blue.  d_normals float64 [capacity_rows, 3] (d2pc_normals_enqueue); d_records 16-byte aligned. */
+int d2pc_ply_normal_records_enqueue(const float *d_xyz, const double *d_normals, const float *d_rgb,
+                                    const uint32_t *d_count, uint32_t capacity_rows, uint8_t *d_records,
+                                    void *stream);
+
 /* f1 -- statistical outlier removal (refine_point_cloud, app.py:252-269: Open3D remove_statistical_outlier(
  * nb_neighbors=20, std_ratio=2.0)) on ONE frame's rows: exact k-nearest neighbours (the point itself
  * included, float64 distances) through a uniform grid, avg[i] = mean of the k distances, keep
@@ -280,6 +286,25 @@ int d2pc_sor_enqueue(const float *d_xyz, const float *d_rgb, const uint32_t *d_c
                      const float *d_bounds, int32_t nb_neighbors, double std_ratio, void *d_scratch,
                      size_t scratch_bytes, float *d_out_xyz, float *d_out_rgb, uint32_t *d_out_index,
                      uint32_t *d_out_count, double *d_stats, void *stream);
+
+/* Point normals (Open3D PointCloud::EstimateNormals with fast_normal_computation, then
+ * OrientNormalsTowardsCameraLocation) on ONE frame's rows, through the same grid as statistical outlier removal:
+ * the knn nearest points (the point itself included, float64 distances, ties ordered by (d2, source row)); with
+ * radius > 0 only points with d2 < radius^2 (Open3D's hybrid search); covariance of those neighbours (identity when
+ * fewer than 3), eigenvector of its smallest eigenvalue (Geometric Tools' robust 3x3 solver, float64), normalised,
+ * (0, 0, 1) when the covariance is zero; with orient != 0 flipped where n . (camera - p) < 0.
+ *   d_bounds       float32 [6] min/max of the rows (emit want_bounds = 1, or d2pc_rows_bounds_enqueue)
+ *   knn            1..64;  radius <= 0: k-NN mode (NaN is refused)
+ *   camera         HOST pointer to 3 doubles, read during the call; may be NULL when orient == 0
+ *   d_scratch      d2pc_normals_scratch_bytes(capacity_rows) bytes, 256-byte aligned
+ *   d_out_normals  float64 [capacity_rows, 3], row i = normal of input row i
+ *   d_out_cov      float64 [capacity_rows, 6] = c00, c01, c02, c11, c12, c22 of every row, or NULL
+ * Argument errors are returned before any launch; the call does not synchronise. */
+int d2pc_normals_scratch_bytes(uint32_t capacity_rows, size_t *bytes);
+int d2pc_normals_enqueue(const float *d_xyz, const uint32_t *d_count, uint32_t capacity_rows,
+                         const float *d_bounds, int32_t knn, double radius, int32_t orient,
+                         const double camera[3], void *d_scratch, size_t scratch_bytes,
+                         double *d_out_normals, double *d_out_cov, void *stream);
 
 #ifdef __cplusplus
 }
