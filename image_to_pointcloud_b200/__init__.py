@@ -11,11 +11,12 @@ from .api import create_depth_preview, depth_preview_bgr, depth_to_point_cloud, 
 from .engine import DENSITY_STEP, BatchStream, EmitResult, FrameEngine, reference_intrinsics, shard_frames
 from .hostpipe import HostFramePipeline, MultiGpuPipeline
 from ._lib import D2pcConfig, D2pcError, D2pcFrameParams, load_library
+from .mesh import TriangleMesh, depth_to_mesh, grid_mesh
 from .normals import estimate_normals
 from .pipeline import point_cloud_stage
 from .refine import refine_point_cloud, statistical_outlier_removal
-from .writers import (las_point_records, ply_vertex_records, preview_lists, preview_rows, save_las, save_ply,
-                      save_point_cloud, save_xyz, xyz_text)
+from .writers import (las_point_records, mesh_ply_bytes, ply_face_records, ply_vertex_records, preview_lists,
+                      preview_rows, save_las, save_mesh_ply, save_ply, save_point_cloud, save_xyz, xyz_text)
 
 __all__ = [
     "depth_to_point_cloud", "depth_to_point_cloud_batch", "create_depth_preview", "depth_preview_bgr", "FrameEngine", "HostFramePipeline", "MultiGpuPipeline",
@@ -23,6 +24,7 @@ __all__ = [
     "D2pcConfig", "D2pcFrameParams", "D2pcError", "load_library",
     "preview_rows", "preview_lists", "xyz_text", "save_xyz", "las_point_records", "save_las", "ply_vertex_records",
     "save_ply", "save_point_cloud", "refine_point_cloud", "statistical_outlier_removal", "point_cloud_stage",
-    "estimate_normals",
+    "estimate_normals", "grid_mesh", "depth_to_mesh", "TriangleMesh", "ply_face_records", "mesh_ply_bytes",
+    "save_mesh_ply",
 ]
 __version__ = "0.1.0"

@@ -22,6 +22,7 @@ constexpr int kXyzMaxLine = 3 * kXyzMaxNumber + 3 * 11 + 6;  // three coordinate
 constexpr int kLasRecordBytes = 26;
 constexpr int kPlyRecordBytes = 27;
 constexpr int kPlyNormalRecordBytes = 51;
+constexpr int kPlyFaceRecordBytes = 13;
 
 // Writes the decimal digits of n (at least one) to out, returns the count.
 D2PC_HD int put_u64(unsigned long long n, char *out) {
@@ -177,6 +178,12 @@ D2PC_HD void ply_normal_record(const float *p, const double *nrm, const float *c
   for (int k = 0; k < 3; ++k) put_f64(o + 8 * k, (double)p[k]);
   for (int k = 0; k < 3; ++k) put_f64(o + 24 + 8 * k, nrm[k]);
   for (int k = 0; k < 3; ++k) o[48 + k] = ply_colour(c[k]);
+}
+
+// Open3D binary PLY face: uchar 3 (property list uchar uint vertex_indices), then three uint32 vertex ids.
+D2PC_HD void ply_face_record(const int32_t *t, uint8_t *o) {
+  o[0] = 3;
+  for (int k = 0; k < 3; ++k) put_le32(o + 1 + 4 * k, (uint32_t)t[k]);
 }
 
 // preview stride of app.py:495-500: points[::stride] with stride = max(1, n // max_preview) when

@@ -9,6 +9,7 @@
 //   LAS 1.2 fmt 2  26-byte records, scaled int32 coordinates, 16-bit colours  -> d2pc_las_records_enqueue
 //   PLY (Open3D)   27-byte records, float64 coordinates, uchar colours        -> d2pc_ply_records_enqueue
 //                  51-byte records, + float64 normals                        -> d2pc_ply_normal_records_enqueue
+//                  13-byte mesh faces, uchar 3 + three uint32 vertex ids     -> d2pc_ply_face_records_enqueue
 // Every entry point works on ONE frame's rows (pointers into the [batch, N, 3] outputs of emit).
 #include "d2pc_device.cuh"
 #include "d2pc_format.h"
@@ -207,6 +208,16 @@ __global__ void __launch_bounds__(kSerThreads) ser_ply_normal_kernel(const float
   });
 }
 
+__global__ void __launch_bounds__(kSerThreads) ser_ply_face_kernel(const int32_t *tri, const uint32_t *count,
+                                                                   uint8_t *records) {
+  ser_records<kPlyFaceRecordBytes>(count, records, [&](uint32_t i, uint8_t *o) {
+    int32_t t[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) t[k] = __ldg(tri + 3 * (size_t)i + k);
+    ply_face_record(t, o);
+  });
+}
+
 // per-axis min / max of the rows (float(points[:, k].min()), app.py:352, 394-399) when emit's fused bounds
 // are not at hand: keys[0..2] = min, keys[3..5] = max (ordered uint32 keys)
 __global__ void ser_bounds_init_kernel(uint32_t *keys) {
@@ -348,6 +359,15 @@ extern "C" int d2pc_ply_normal_records_enqueue(const float *d_xyz, const double 
   if (capacity_rows == 0 || ((uintptr_t)d_records & 15u) != 0) return D2PC_ERR_INVALID_ARGUMENT;
   ser_ply_normal_kernel<<<ser_tiles(capacity_rows), kSerThreads, 0, (cudaStream_t)stream>>>(d_xyz, d_normals, d_rgb,
                                                                                             d_count, d_records);
+  D2PC_CHECK_LAUNCH();
+  return D2PC_OK;
+}
+
+extern "C" int d2pc_ply_face_records_enqueue(const int32_t *d_tri, const uint32_t *d_tri_count, uint32_t capacity,
+                                             uint8_t *d_records, void *stream) {
+  if (!d_tri || !d_tri_count || !d_records) return D2PC_ERR_INVALID_ARGUMENT;
+  if (capacity == 0 || ((uintptr_t)d_records & 15u) != 0) return D2PC_ERR_INVALID_ARGUMENT;
+  ser_ply_face_kernel<<<ser_tiles(capacity), kSerThreads, 0, (cudaStream_t)stream>>>(d_tri, d_tri_count, d_records);
   D2PC_CHECK_LAUNCH();
   return D2PC_OK;
 }

@@ -1,0 +1,162 @@
+"""Row m1: a triangle mesh of one frame on the device, from the image lattice its points come from.
+
+The unmasked emit row ``i = r * C + c`` comes from pixel ``(r * step, c * step)`` of an ``R x C = ceil(H / step) x
+ceil(W / step)`` lattice, so every point's neighbours are known without a search.  Each lattice quad is split into
+two triangles along its shorter diagonal; triangles that are degenerate, face away from the camera, or are seen at
+more than ``max_angle`` degrees from their normal (the ones that bridge a depth discontinuity) are dropped.  This is
+the standard depth-image triangulation, not the reference's Poisson / BPA mesh builder (backend/app.py:271-308): it
+runs in milliseconds and is deterministic, and the spec is our own (DESIGN.md, row m1).
+
+    mesh = depth_to_mesh(image, depth, density="medium", z_range=(0.5, 9.5), refine=True)
+    save_mesh_ply(mesh, "scene")                          # outputs/scene.ply, Open3D's binary layout
+
+Run by ``d2pc_grid_mesh_enqueue``; vertex normals follow Open3D's ``ComputeVertexNormals`` (float64).
+"""
+from __future__ import annotations
+
+import ctypes as C
+import math
+from typing import NamedTuple, Optional
+
+import numpy as np
+import torch
+
+from . import _lib
+from ._lib import check
+from .api import _engine_for, _image_channels, check_depth_dtype
+from .engine import DENSITY_STEP
+from .refine import statistical_outlier_removal
+from .writers import _device_rows, _stream
+
+
+class TriangleMesh(NamedTuple):
+    vertices: object               # float32 [V, 3]
+    colors: object                 # float32 [V, 3] (0..255, like the point cloud's colours)
+    triangles: object              # int32 [T, 3] vertex ids, ordered by lattice quad
+    vertex_normals: Optional[object]   # float64 [V, 3] or None
+    vertex_rows: object            # int64 [V] lattice row of every vertex
+
+
+def _cos2(max_angle) -> float:
+    a = float(max_angle)
+    if not 0.0 < a <= 90.0:
+        raise ValueError("max_angle must be in (0, 90] degrees")
+    c = math.cos(math.radians(a))
+    return c * c
+
+
+def _max_edge(max_edge) -> float:
+    if max_edge is None:
+        return 0.0
+    e = float(max_edge)
+    if not (np.isfinite(e) and e > 0.0):
+        raise ValueError("max_edge must be a positive finite number or None")
+    return e
+
+
+def grid_mesh(points, colors, lattice_shape, *, keep=None, max_edge=None, max_angle: float = 85.0,
+              remove_unreferenced: bool = True, compute_normals: bool = True, device=None,
+              return_device: bool = False) -> TriangleMesh:
+    """Triangle mesh of the ``lattice_shape = (R, C)`` lattice rows ``points`` / ``colors`` (float32 [R*C, 3]).
+
+    A row is a vertex only when ``keep`` (bool / uint8 [R*C], optional) holds and its coordinates are finite; with
+    ``remove_unreferenced`` only rows used by a kept triangle stay.  ``max_edge`` drops triangles with a longer edge,
+    ``max_angle`` (degrees, (0, 90]) those seen at a more grazing angle.  NumPy arrays, or CUDA tensors with
+    ``return_device``."""
+    R, Cc = int(lattice_shape[0]), int(lattice_shape[1])
+    if R < 1 or Cc < 1 or R * Cc >= 2 ** 31:
+        raise ValueError("lattice_shape must be (R, C) with R, C >= 1 and R * C < 2^31")
+    cos2, me = _cos2(max_angle), _max_edge(max_edge)
+    lib = _lib.load_library()
+    xyz, rgb, _, n = _device_rows(points, colors, device)
+    if n != R * Cc:
+        raise ValueError(f"{n} rows do not form a {R} x {Cc} lattice")
+    dev = xyz.device
+    with torch.cuda.device(dev):
+        keep_t = None
+        if keep is not None:
+            keep_t = keep if isinstance(keep, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(keep))
+            keep_t = keep_t.to(dev).reshape(-1)
+            if keep_t.numel() != n:
+                raise ValueError("keep must have one entry per lattice row")
+            keep_t = (keep_t != 0).to(torch.uint8).contiguous()
+        nb = C.c_size_t(0)
+        check(lib.d2pc_grid_mesh_scratch_bytes(R, Cc, C.byref(nb)), "d2pc_grid_mesh_scratch_bytes")
+        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+        vxyz = torch.empty((n, 3), dtype=torch.float32, device=dev)
+        vrgb = torch.empty((n, 3), dtype=torch.float32, device=dev)
+        vrow = torch.empty(n, dtype=torch.int32, device=dev)
+        vnrm = torch.empty((n, 3), dtype=torch.float64, device=dev) if compute_normals else None
+        tri = torch.empty((max(2 * (R - 1) * (Cc - 1), 1), 3), dtype=torch.int32, device=dev)
+        counts = torch.zeros(2, dtype=torch.int32, device=dev)   # vertices, triangles
+        flags = (_lib.MESH_REMOVE_UNREFERENCED if remove_unreferenced else 0) | \
+            (_lib.MESH_NORMALS if compute_normals else 0)
+        check(lib.d2pc_grid_mesh_enqueue(xyz.data_ptr(), rgb.data_ptr(), keep_t.data_ptr() if keep_t is not None else None,
+                                         R, Cc, me, cos2, flags, scratch.data_ptr(), scratch.numel(), vxyz.data_ptr(),
+                                         vrgb.data_ptr(), vrow.data_ptr(), vnrm.data_ptr() if vnrm is not None else None,
+                                         counts.data_ptr(), tri.data_ptr(), counts.data_ptr() + 4, _stream(dev)),
+              "d2pc_grid_mesh_enqueue")
+        nv, nt = (int(v) for v in counts.cpu())
+        mesh = TriangleMesh(vxyz[:nv], vrgb[:nv], tri[:nt], vnrm[:nv] if vnrm is not None else None,
+                            vrow[:nv].to(torch.int64))
+        if return_device:
+            return mesh
+        return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in mesh))
+
+
+def lattice_shape(img_h: int, img_w: int, density: str):
+    """(R, C) of the emit lattice: ceil(H / step) x ceil(W / step)."""
+    s = DENSITY_STEP[density]
+    return -(-int(img_h) // s), -(-int(img_w) // s)
+
+
+def refined_keep(xyz: torch.Tensor, keep: Optional[torch.Tensor], nb_neighbors: int, std_ratio: float) -> torch.Tensor:
+    """Statistical outlier removal on the kept lattice rows (all rows when ``keep`` is None), its kept index scattered
+    back into a uint8 lattice mask: the rows ``refine_point_cloud`` keeps of the same cloud."""
+    n = int(xyz.shape[0])
+    rows = torch.arange(n, device=xyz.device) if keep is None else torch.nonzero(keep).reshape(-1)
+    out = torch.zeros(n, dtype=torch.uint8, device=xyz.device)
+    if rows.numel() > 0:
+        _, _, idx, _ = statistical_outlier_removal(xyz[rows].contiguous(), None, nb_neighbors, std_ratio,
+                                                   return_device=True)
+        out[rows[idx.to(torch.int64)]] = 1
+    return out
+
+
+def depth_to_mesh(image: np.ndarray, depth: np.ndarray, density: str = "medium", invert: bool = True,
+                  depth_scale: float = 10.0, smooth: bool = False, smooth_ksize: int = 5, fov: Optional[float] = None,
+                  *, z_range=None, refine: bool = False, nb_neighbors: int = 20, std_ratio: float = 2.0,
+                  max_edge=None, max_angle: float = 85.0, remove_unreferenced: bool = True,
+                  compute_normals: bool = True, device=None, return_device: bool = False) -> TriangleMesh:
+    """Mesh of one (image, depth) pair in one device-resident pass: the unmasked emit of ``depth_to_point_cloud``
+    (same positional arguments), ``z_range`` as a mask on the lattice (the float32 rule of the depth-range mask),
+    with ``refine`` statistical outlier removal of the remaining rows (``nb_neighbors``, ``std_ratio``), then
+    ``grid_mesh``.  The vertices are the points ``depth_to_point_cloud(..., z_range=z_range)`` followed by
+    ``refine_point_cloud`` would keep (those a kept triangle uses, with ``remove_unreferenced``)."""
+    DENSITY_STEP[density]  # KeyError first, like the reference
+    if z_range is not None and len(z_range) != 2:
+        raise ValueError("z_range must be (z_min, z_max)")
+    _cos2(max_angle), _max_edge(max_edge)   # argument errors before any device work
+    img_h, img_w = image.shape[:2]
+    dep_h, dep_w = depth.shape[:2]
+    check_depth_dtype(depth, int(img_h), int(img_w))
+    img_c = _image_channels(image)
+    eng = _engine_for(int(img_h), int(img_w), img_c, int(dep_h), int(dep_w), device)
+    dev = eng.device
+    cfg = eng.make_config(density=density, invert=invert, depth_scale=float(depth_scale), fov=fov)
+    with eng._staging["lock"], torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev)
+        d = torch.from_numpy(np.ascontiguousarray(depth, dtype=np.float32).reshape(1, dep_h, dep_w)).to(dev)
+        im = torch.from_numpy(np.ascontiguousarray(image).reshape(1, img_h, img_w, -1)).to(dev) if img_c >= 3 else None
+        res = eng.process(cfg, d, im, stream=stream, smooth_ksize=(smooth_ksize if smooth else None))
+        n = eng.points_per_frame(cfg)
+        xyz, rgb = res.xyz[0, :n], res.rgb[0, :n]
+        keep = None
+        if z_range is not None:   # z32 >= f32(z_min) and z32 <= f32(z_max)
+            z = xyz[:, 2]
+            keep = ((z >= float(np.float32(z_range[0]))) & (z <= float(np.float32(z_range[1])))).to(torch.uint8)
+        if refine:
+            keep = refined_keep(xyz, keep, nb_neighbors, std_ratio)
+        return grid_mesh(xyz, rgb, lattice_shape(img_h, img_w, density), keep=keep, max_edge=max_edge,
+                         max_angle=max_angle, remove_unreferenced=remove_unreferenced,
+                         compute_normals=compute_normals, return_device=return_device)

@@ -4,6 +4,7 @@
     depth_to_point_cloud (:468-476) -> refine_point_cloud (:479) -> preview decimation (:495-506)
     -> save_point_cloud (:537) -> generate_gis_metadata bounds (:393-400)
     [-> estimate_normals, the mesh builder's first step (:271-308), with normals=True]
+    [-> grid_mesh of the refined lattice rows, the mesh PLY (row m1), with mesh=True]
 
 Called as separate drop-ins, those steps move the cloud across PCIe five times (down after the stage, up
 and down around the refinement, up again for the writer).  Here the image and the depth map go up once,
@@ -24,6 +25,7 @@ from . import _lib, writers
 from ._lib import check
 from .api import _engine_for, _image_channels, _to_host, bounds_dict, check_depth_dtype
 from .engine import DENSITY_STEP
+from .mesh import _cos2, _max_edge, grid_mesh, lattice_shape
 from .normals import estimate_normals
 from .refine import statistical_outlier_removal
 
@@ -33,14 +35,20 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
                       refine: bool = True, nb_neighbors: int = 20, std_ratio: float = 2.0,
                       output_format: Optional[str] = "ply", filename: Optional[str] = None,
                       max_preview: int = writers.MAX_PREVIEW, return_arrays: bool = True, normals: bool = False,
-                      normals_knn: int = 30, device=None) -> dict:
+                      normals_knn: int = 30, mesh: bool = False, mesh_max_angle: float = 85.0, mesh_max_edge=None,
+                      device=None) -> dict:
     """Returns a dict with ``points`` / ``colors`` (host float32 [M,3], if ``return_arrays``), ``point_count``,
     ``preview_points`` / ``preview_colors`` (nested lists as app.py:505-506), ``bounds`` (app.py:393-400),
     and either ``filepath`` (``filename`` given: the file the reference's writer would have put into
     outputs/<filename>.<ext>) or ``file_bytes`` (its content).  With ``normals`` the refined rows' normals
     (``estimate_normals(points, knn=normals_knn)``, float64 [M,3]) are computed on the device, returned as
-    ``normals`` (if ``return_arrays``) and written into a PLY file."""
+    ``normals`` (if ``return_arrays``) and written into a PLY file.  With ``mesh`` the (refined) lattice rows are
+    also meshed (``grid_mesh(..., max_angle=mesh_max_angle, max_edge=mesh_max_edge)``, vertex normals included):
+    ``mesh_vertex_count``, ``mesh_triangle_count`` and either ``mesh_filepath`` (outputs/<filename>_mesh.ply) or
+    ``mesh_file_bytes``."""
     DENSITY_STEP[density]  # KeyError first, like the reference
+    if mesh:   # mesh argument errors before any device work
+        _cos2(mesh_max_angle), _max_edge(mesh_max_edge)
     lib = _lib.load_library()
     img_h, img_w = image.shape[:2]
     dep_h, dep_w = depth.shape[:2]
@@ -56,8 +64,9 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
         res = eng.process(cfg, d, im, stream=stream, smooth_ksize=(smooth_ksize if smooth else None))
         n = int(res.count.cpu()[0])
         xyz, rgb = res.xyz[0, :n], res.rgb[0, :n]
+        lat_xyz, lat_rgb, kept = xyz, rgb, None   # the emit rows are the unmasked lattice
         if refine and n > 0:
-            xyz, rgb, _, _ = statistical_outlier_removal(xyz, rgb, nb_neighbors, std_ratio, return_device=True)
+            xyz, rgb, kept, _ = statistical_outlier_removal(xyz, rgb, nb_neighbors, std_ratio, return_device=True)
         m = int(xyz.shape[0])
         out = {"point_count": m}
         nrm = estimate_normals(xyz, knn=normals_knn, return_device=True) if normals else None
@@ -97,4 +106,16 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
                 out["filepath"] = path
             else:
                 out["file_bytes"] = head + rec.tobytes()
+        if mesh:
+            keep = None
+            if kept is not None:
+                keep = torch.zeros(n, dtype=torch.uint8, device=dev)
+                keep[kept.to(torch.int64)] = 1
+            msh = grid_mesh(lat_xyz, lat_rgb, lattice_shape(img_h, img_w, density), keep=keep, max_edge=mesh_max_edge,
+                            max_angle=mesh_max_angle, return_device=True)
+            out["mesh_vertex_count"], out["mesh_triangle_count"] = len(msh.vertices), len(msh.triangles)
+            if filename is not None:
+                out["mesh_filepath"] = writers.save_mesh_ply(msh, f"{filename}_mesh")
+            else:
+                out["mesh_file_bytes"] = writers.mesh_ply_bytes(msh)
         return out

@@ -5,6 +5,7 @@ with the per-point work moved to the GPU.
     save_xyz(points, colors, filename)       app.py:379-389   ASCII "%.6f %.6f %.6f %d %d %d" lines
     save_las(points, colors, filename)       app.py:343-377   LAS 1.2, point format 2 (scale 0.01, offset = min)
     save_ply(points, colors, filename)       app.py:329-341   Open3D binary little-endian PLY (normals=: with nx, ny, nz)
+    save_mesh_ply(mesh, filename)            (row m1)         Open3D write_triangle_mesh binary PLY of a TriangleMesh
     save_point_cloud(points, colors, format, filename)   app.py:310-327   the dispatcher
 
 Same signatures and return values (the file path under ``outputs/``) as the reference.  ``points`` /
@@ -36,6 +37,7 @@ logger = logging.getLogger(__name__)
 LAS_RECORD_BYTES = 26
 PLY_RECORD_BYTES = 27
 PLY_NORMAL_RECORD_BYTES = 51
+PLY_FACE_RECORD_BYTES = 13
 MAX_PREVIEW = 20000  # app.py:496
 
 
@@ -240,6 +242,67 @@ def save_ply(points, colors, filename: str, device=None, normals=None) -> str:
     with open(filepath, "wb") as f:
         f.write(header.format(n=len(rec)).encode("ascii"))
         f.write(rec.tobytes())
+    return filepath
+
+
+# ---- mesh PLY (Open3D write_triangle_mesh, row m1) --------------------------------------------
+# the vertex header of the point-cloud PLY plus Open3D's face element
+PLY_FACE_ELEMENT = "element face {m}\nproperty list uchar uint vertex_indices\n"
+PLY_MESH_HEADER = PLY_HEADER.replace("end_header\n", PLY_FACE_ELEMENT + "end_header\n")
+PLY_MESH_NORMAL_HEADER = PLY_NORMAL_HEADER.replace("end_header\n", PLY_FACE_ELEMENT + "end_header\n")
+
+
+def ply_face_records(triangles, device=None) -> np.ndarray:
+    """-> uint8 [t, 13]: uchar 3 and the three vertex ids as uint32 per triangle (int32 [t, 3] in)."""
+    lib = _lib.load_library()
+    if isinstance(triangles, torch.Tensor):
+        tri = triangles
+    else:
+        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+        tri = torch.from_numpy(np.ascontiguousarray(triangles, dtype=np.int32).reshape(-1, 3)).to(dev)
+    if tri.dtype != torch.int32 or tri.dim() != 2 or tri.shape[1] != 3:
+        raise ValueError("triangles must be int32 [T, 3]")
+    t = int(tri.shape[0])
+    if t == 0:
+        return np.zeros((0, PLY_FACE_RECORD_BYTES), np.uint8)
+    dev = tri.device
+    with torch.cuda.device(dev):
+        tri = tri.contiguous()
+        cnt = torch.tensor([t], dtype=torch.int32, device=dev)
+        rec = torch.empty(t * PLY_FACE_RECORD_BYTES + 16, dtype=torch.uint8, device=dev)
+        check(lib.d2pc_ply_face_records_enqueue(tri.data_ptr(), cnt.data_ptr(), t, rec.data_ptr(), _stream(dev)),
+              "d2pc_ply_face_records_enqueue")
+        host = torch.empty(t * PLY_FACE_RECORD_BYTES, dtype=torch.uint8, pin_memory=True)
+        host.copy_(rec[:t * PLY_FACE_RECORD_BYTES])
+        return host.numpy().reshape(t, PLY_FACE_RECORD_BYTES)
+
+
+def _mesh_ply_parts(mesh, device=None):
+    """-> (header bytes, vertex records, face records) of a TriangleMesh (NumPy arrays or CUDA tensors)."""
+    nrm = mesh.vertex_normals
+    dev = mesh.vertices.device if isinstance(mesh.vertices, torch.Tensor) else device
+    vrec = ply_vertex_records(mesh.vertices, mesh.colors, dev, normals=nrm)
+    frec = ply_face_records(mesh.triangles, dev)
+    header = PLY_MESH_HEADER if nrm is None else PLY_MESH_NORMAL_HEADER
+    return header.format(n=len(vrec), m=len(frec)).encode("ascii"), vrec, frec
+
+
+def mesh_ply_bytes(mesh, device=None) -> bytes:
+    """The binary PLY Open3D's ``write_triangle_mesh`` writes for the mesh: vertices (float64 x, y, z, then nx, ny,
+    nz when the mesh has normals, uchar red, green, blue) and 13-byte faces."""
+    head, vrec, frec = _mesh_ply_parts(mesh, device)
+    return head + vrec.tobytes() + frec.tobytes()
+
+
+def save_mesh_ply(mesh, filename: str, device=None) -> str:
+    """Write the mesh as ``outputs/<filename>.ply`` (``mesh_ply_bytes``) and return the path, like ``save_ply``."""
+    filepath = f"outputs/{filename}.ply"
+    head, vrec, frec = _mesh_ply_parts(mesh, device)
+    Path("outputs").mkdir(exist_ok=True)
+    with open(filepath, "wb") as f:
+        f.write(head)
+        f.write(vrec)   # straight from the pinned buffers (either may be empty)
+        f.write(frec)
     return filepath
 
 

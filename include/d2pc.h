@@ -34,6 +34,10 @@
  *   f3 preview stride (:495-506), save_xyz/las/ply (:329-389) -> d2pc_preview_rows_enqueue,
  *                                                               d2pc_xyz_text_*, d2pc_las_records_enqueue,
  *                                                               d2pc_ply_records_enqueue
+ *   n1 point normals (the mesh builder's first step, :271-308) -> d2pc_normals_enqueue
+ *   m1 lattice mesh (our own spec; the reference meshes with
+ *      Poisson / BPA, :271-308)                                -> d2pc_grid_mesh_enqueue,
+ *                                                               d2pc_ply_face_records_enqueue
  */
 #ifndef D2PC_H_
 #define D2PC_H_
@@ -305,6 +309,40 @@ int d2pc_normals_enqueue(const float *d_xyz, const uint32_t *d_count, uint32_t c
                          const float *d_bounds, int32_t knn, double radius, int32_t orient,
                          const double camera[3], void *d_scratch, size_t scratch_bytes,
                          double *d_out_normals, double *d_out_cov, void *stream);
+
+/* m1 -- triangle mesh of ONE frame's lattice: the rows of an unmasked emit (row i = r * cols + c of a rows x cols
+ * lattice, i.e. ceil(H / step) x ceil(W / step)).  A row is a vertex candidate when d_keep[i] != 0 (or d_keep is
+ * NULL) and its three coordinates are finite.  Quad (r, c) has corners a (r, c), b (r, c+1), p (r+1, c), d (r+1, c+1):
+ * with four valid corners it is split along a-d into (a, p, d), (a, d, b) when d2(a, d) <= d2(b, p), else along b-p
+ * into (a, p, b), (b, p, d); with three valid corners it gives the triangle of those three (in this winding).  A
+ * triangle is kept when, in float64 with n = (p1 - p0) x (p2 - p0) and s = (p0 + p1) + p2: n.n > 0, n.s < 0 (it
+ * faces the camera), (n.s)^2 >= cos2 (n.n)(s.s) (it is not grazing: depth discontinuities are dropped), and, with
+ * max_edge > 0, every edge has d2 <= max_edge^2.
+ *   flags          D2PC_MESH_REMOVE_UNREFERENCED: only rows used by a kept triangle become vertices (else every valid
+ *                  row); D2PC_MESH_NORMALS: vertex normals (Open3D ComputeVertexNormals: the unnormalised n of the
+ *                  adjacent kept triangles summed in ascending triangle order, normalised; (0, 0, 1) for a zero sum)
+ *   cos2           cos(max_angle)^2 in [0, 1];  max_edge <= 0: no edge limit (NaN / inf are refused)
+ *   d_scratch      d2pc_grid_mesh_scratch_bytes(rows, cols) bytes, 256-byte aligned
+ *   d_vtx_xyz/rgb  float32 [rows * cols, 3]; d_vtx_row int32 [rows * cols] lattice row of every vertex;
+ *                  d_vtx_normals float64 [rows * cols, 3] (needed with D2PC_MESH_NORMALS, else may be NULL);
+ *                  d_vtx_count uint32 [1]; vertices in lattice order
+ *   d_tri          int32 [2 (rows - 1)(cols - 1), 3] vertex ids (may be NULL when rows or cols is 1);
+ *                  d_tri_count uint32 [1]; triangles ordered by quad, (a, p, *) first
+ * rows * cols must be below 2^31.  Argument errors are returned before any launch; the call does not synchronise
+ * and the result repeats bit for bit. */
+enum { D2PC_MESH_REMOVE_UNREFERENCED = 1, D2PC_MESH_NORMALS = 2 };
+int d2pc_grid_mesh_scratch_bytes(uint32_t rows, uint32_t cols, size_t *bytes);
+int d2pc_grid_mesh_enqueue(const float *d_xyz, const float *d_rgb, const uint8_t *d_keep, uint32_t rows,
+                           uint32_t cols, double max_edge, double cos2, uint32_t flags, void *d_scratch,
+                           size_t scratch_bytes, float *d_vtx_xyz, float *d_vtx_rgb, int32_t *d_vtx_row,
+                           double *d_vtx_normals, uint32_t *d_vtx_count, int32_t *d_tri, uint32_t *d_tri_count,
+                           void *stream);
+
+/* Binary little-endian PLY faces as Open3D's write_triangle_mesh writes them ("property list uchar uint
+ * vertex_indices"), 13 bytes each: uchar 3, then three uint32 vertex ids.  d_tri int32 [capacity, 3] with
+ * *d_tri_count <= capacity rows in use; d_records 16-byte aligned, capacity * 13 bytes. */
+int d2pc_ply_face_records_enqueue(const int32_t *d_tri, const uint32_t *d_tri_count, uint32_t capacity,
+                                  uint8_t *d_records, void *stream);
 
 #ifdef __cplusplus
 }
