@@ -17,9 +17,11 @@
 //   flags  u8[N]      1 = this row is a representative
 //   * colours are the integral 0..255 floats emit writes: their sums are exact integers, two packed
 //     64-bit adds carry count, r, g and b (N < 2^24 rows keeps every 32-bit field from overflowing);
-//   * coordinates are accumulated as 64-bit fixed point of (p - vmin) with a power-of-two scale
-//     chosen per frame so that N * extent * scale < 2^62: integer adds are associative, so the
-//     means are deterministic (run-to-run identical) and within 2^-38 * extent of the float64 sums.
+//   * coordinates are accumulated as 64-bit fixed point of (p - bmin), bmin = the frame's min_xyz, with a
+//     power-of-two scale chosen per frame from the cloud's own extent E = max over axes of (bmax - bmin), so that
+//     N * E * scale < 2^62: integer adds are associative, so the means are deterministic (run-to-run identical)
+//     and within 2^-38 * E of the float64 means.  The origin is NOT vmin: vmin = bmin - vs/2 would tie the
+//     quantum to the voxel size, and a voxel much larger than the cloud would then lose the means.
 //   * insert: one row per lane; rows that share a voxel with their left neighbour form a run that is summed in
 //     registers by a segmented warp scan (raster neighbours share voxels in smooth scenes); the run's last lane
 //     probes.  A read-only probe comes first, so members of an existing voxel never write their own slot.
@@ -28,6 +30,8 @@
 // Against the first design (64-byte hash entries, 1 GB table for a 4K frame, every access a random DRAM
 // read-modify-write) the random traffic drops to 4-byte entries in an L2-resident table.
 #include <stdlib.h>
+
+#include <cmath>
 
 #include "d2pc_device.cuh"
 
@@ -48,7 +52,8 @@ struct __align__(256) VoxHeader {
   uint32_t n_out;            // output rows of the frame being processed
   uint32_t done;             // extract CTAs finished (ticket for the final count)
   uint32_t frame_cap;        // slots used for the current frame (2 * rows, >= 1024, <= cap)
-  double vmin[3];
+  double vmin[3];            // voxel index origin: bmin - vs/2
+  double origin[3];          // fixed-point origin: bmin
   double scale;              // fixed-point scale (power of two)
   int32_t bad;               // table was not initialised
 };
@@ -112,14 +117,16 @@ __global__ void vox_begin_kernel(VoxTable t, const uint32_t *count, const float 
   const double half = vs * 0.5;
   double ext = 0.0;
   for (int c = 0; c < 3; ++c) {
-    const double vmin = (double)bounds[c] - half;
-    h->vmin[c] = vmin;
-    const double e = (double)bounds[3 + c] - vmin;
+    const double bmin = (double)bounds[c];
+    h->vmin[c] = bmin - half;
+    h->origin[c] = bmin;
+    const double e = (double)bounds[3 + c] - bmin;   // float32 bounds: finite, at most 2 * FLT_MAX
     if (e > ext) ext = e;
   }
-  // N * ext * scale < 2^62  with  N <= 2^24: scale = 2^(38 - ceil(log2(ext)))
+  // N * ext * scale < 2^62  with  N <= 2^24: scale = 2^(38 - ceil(log2(ext))); each term is rounded by at most
+  // 0.5 / scale = 2^(ex - 39) <= 2^-38 * ext
   int ex = 0;
-  if (ext > 0.0 && ext < 1.0e300) frexp(ext, &ex);  // ext = m * 2^ex, 0.5 <= m < 1
+  if (ext > 0.0) frexp(ext, &ex);  // ext = m * 2^ex, 0.5 <= m < 1
   h->scale = ldexp(1.0, 38 - ex);
   const unsigned long long m2 = 2ull * (unsigned long long)*count;
   h->frame_cap = (uint32_t)(m2 < 1024ull ? 1024ull : (m2 > t.cap ? t.cap : m2));
@@ -264,6 +271,7 @@ __global__ void __launch_bounds__(kVoxThreads, 4) vox_insert_kernel(VoxTable t, 
   const uint32_t tile_base = blockIdx.x * (uint32_t)kVoxTile;
   if (tile_base >= M || t.hdr->bad) return;
   const double vmin0 = t.hdr->vmin[0], vmin1 = t.hdr->vmin[1], vmin2 = t.hdr->vmin[2];
+  const double org0 = t.hdr->origin[0], org1 = t.hdr->origin[1], org2 = t.hdr->origin[2];
   const double scale = t.hdr->scale;
   const uint32_t frame_cap = t.hdr->frame_cap;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -296,9 +304,9 @@ __global__ void __launch_bounds__(kVoxThreads, 4) vox_insert_kernel(VoxTable t, 
                   (unsigned long long)i2d;
         run.cnt_r = (1ull << 32) | (unsigned long long)(uint32_t)c0;
         run.g_b = ((unsigned long long)(uint32_t)c1 << 32) | (unsigned long long)(uint32_t)c2;
-        run.sx = (unsigned long long)__double2ll_rn(o0 * scale);
-        run.sy = (unsigned long long)__double2ll_rn(o1 * scale);
-        run.sz = (unsigned long long)__double2ll_rn(o2 * scale);
+        run.sx = (unsigned long long)__double2ll_rn(((double)x0 - org0) * scale);
+        run.sy = (unsigned long long)__double2ll_rn(((double)x1 - org1) * scale);
+        run.sz = (unsigned long long)__double2ll_rn(((double)x2 - org2) * scale);
       } else {
         *err = 1;  // "voxel_size is too small." (or non-finite coordinates)
       }
@@ -394,7 +402,7 @@ __global__ void __launch_bounds__(kVoxThreads, 3) vox_extract_kernel(VoxTable t,
   if (!failed && mine) {
     uint32_t j = s_base + woff + incl - mine;
     const double inv_scale = 1.0 / t.hdr->scale;  // power of two: exact
-    const double vmin0 = t.hdr->vmin[0], vmin1 = t.hdr->vmin[1], vmin2 = t.hdr->vmin[2];
+    const double org0 = t.hdr->origin[0], org1 = t.hdr->origin[1], org2 = t.hdr->origin[2];
     unsigned long long w[4][6];
 #pragma unroll
     for (int k = 0; k < 4; ++k) {  // all loads of the thread's representatives in flight together
@@ -414,9 +422,9 @@ __global__ void __launch_bounds__(kVoxThreads, 3) vox_extract_kernel(VoxTable t,
       // (div_by_const_fast: numerators are >= 0 and finite, n is a small integer -- same bits as a / n)
       const double rn = 1.0 / n;
       float *ox = oxyz + 3 * (size_t)j, *oc = orgb + 3 * (size_t)j;
-      stg_stream_f1(ox + 0, (float)(vmin0 + div_by_const_fast((double)(long long)sx * inv_scale, n, rn)));
-      stg_stream_f1(ox + 1, (float)(vmin1 + div_by_const_fast((double)(long long)sy * inv_scale, n, rn)));
-      stg_stream_f1(ox + 2, (float)(vmin2 + div_by_const_fast((double)(long long)sz * inv_scale, n, rn)));
+      stg_stream_f1(ox + 0, (float)(org0 + div_by_const_fast((double)(long long)sx * inv_scale, n, rn)));
+      stg_stream_f1(ox + 1, (float)(org1 + div_by_const_fast((double)(long long)sy * inv_scale, n, rn)));
+      stg_stream_f1(ox + 2, (float)(org2 + div_by_const_fast((double)(long long)sz * inv_scale, n, rn)));
       stg_stream_f1(oc + 0, (float)div_by_const_fast((double)(uint32_t)cnt_r, n, rn));
       stg_stream_f1(oc + 1, (float)div_by_const_fast((double)(uint32_t)(g_b >> 32), n, rn));
       stg_stream_f1(oc + 2, (float)div_by_const_fast((double)(uint32_t)g_b, n, rn));
@@ -473,7 +481,7 @@ extern "C" int d2pc_voxel_enqueue(const D2pcConfig *cfg, double voxel_size, cons
                                   void *stream) {
   int rc = validate_config(cfg);
   if (rc) return rc;
-  if (!(voxel_size > 0.0)) return D2PC_ERR_INVALID_ARGUMENT;
+  if (!(std::isfinite(voxel_size) && voxel_size > 0.0)) return D2PC_ERR_INVALID_ARGUMENT;
   if (!d_xyz || !d_rgb || !d_count || !d_bounds || !d_table || !d_vox_xyz || !d_vox_rgb || !d_vox_count ||
       !d_vox_error)
     return D2PC_ERR_INVALID_ARGUMENT;

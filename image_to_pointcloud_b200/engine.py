@@ -99,6 +99,7 @@ class FrameEngine:
             self._any_host = torch.zeros(1, dtype=torch.int32, pin_memory=True)
         assert self.workspace.data_ptr() % 256 == 0
         self._voxel_table = None
+        self._voxel_rows = None   # rows per frame the voxel table was last initialised for
         self._smooth_scratch = None
         self._path = None
 
@@ -342,13 +343,19 @@ class FrameEngine:
             raise ValueError("voxel_downsample needs an emit with want_bounds=True")
         if not voxel_size > 0:
             raise ValueError("voxel_size <= 0.")
+        if not np.isfinite(voxel_size):
+            raise ValueError("voxel_size must be finite.")
         nbytes = C.c_size_t(0)
         check(self.lib.d2pc_voxel_table_bytes(C.byref(cfg), C.byref(nbytes)), "d2pc_voxel_table_bytes")
+        n = self.points_per_frame(cfg)
         with torch.cuda.device(self.device):
             if self._voxel_table is None or self._voxel_table.numel() < nbytes.value:
                 self._voxel_table = torch.empty(int(nbytes.value), dtype=torch.uint8, device=self.device)
+                self._voxel_rows = None
+            if self._voxel_rows != n:   # the table's layout depends on the rows per frame (density)
                 self._call("d2pc_voxel_table_init", C.byref(cfg), self._voxel_table.data_ptr(),
                            self._voxel_table.numel(), self._stream(stream))
+                self._voxel_rows = n
             vxyz = torch.empty_like(res.xyz)
             vrgb = torch.empty_like(res.rgb)
             vidx = torch.empty(res.xyz.shape, dtype=torch.int32, device=self.device) if want_index else None

@@ -207,18 +207,24 @@ int d2pc_preview_enqueue(const D2pcConfig *cfg, const float *d_depth, void *d_wo
 
 /* ax-2 voxel-grid down-sampling of each frame's emitted rows (Open3D VoxelDownSample semantics:
  * vmin = min_xyz - vs/2, idx = floor((p - vmin)/vs) on float64 copies, mean of members).
+ *   voxel_size    finite and > 0 (else D2PC_ERR_INVALID_ARGUMENT before any launch)
  *   d_xyz/d_rgb/d_count/d_bounds  outputs of d2pc_emit_enqueue (want_bounds = 1), row stride N;
  *                 colours must be the integral 0..255 values emit writes (their sums are kept exact)
  *   d_table       scratch of d2pc_voxel_table_bytes() bytes, 256-byte aligned, on which
- *                 d2pc_voxel_table_init() has run once after allocation: a table of 4-byte slots (8-bit
- *                 fingerprint | 24-bit row of the voxel's representative row, small enough to stay in L2), and
- *                 per-row keys, accumulators and flags that are only touched in row order (csrc/d2pc_voxel.cu).
- *                 Cleared per frame by the call itself.
+ *                 d2pc_voxel_table_init() has run with a config of the same rows per frame N: a table of
+ *                 4-byte slots (8-bit fingerprint | 24-bit row of the voxel's representative row, small enough
+ *                 to stay in L2), and per-row keys, accumulators and flags that are only touched in row order
+ *                 (csrc/d2pc_voxel.cu).  The layout depends on N, so initialise again whenever the config's N
+ *                 changes (another density); otherwise the frames fail with error 2.  Cleared per frame by the
+ *                 call itself.
  *   d_vox_xyz/rgb float32 [batch, N, 3]; d_vox_idx int32 [batch, N, 3] or NULL;
  *   d_vox_count   uint32 [batch]; d_vox_error int32 [batch] (1 = index overflow, >= 2^21;
  *                 2 = table not initialised)
- * Coordinates are summed as 64-bit fixed point of (p - vmin) (deterministic, within 2^-38 of the
- * frame's extent of the float64 sums); frames of 2^24 rows or more return D2PC_ERR_UNSUPPORTED. */
+ * Coordinates are summed as 64-bit fixed point of (p - min_xyz), scaled to the cloud's extent
+ * E = max over axes of (max_xyz - min_xyz): the means are deterministic and within 2^-38 * E (plus the
+ * float32 rounding of the result) of the float64 means, whatever the voxel size.  Colour means are exact
+ * (correctly rounded quotients of exact integer sums).  Frames of 2^24 rows or more return
+ * D2PC_ERR_UNSUPPORTED. */
 int d2pc_voxel_table_bytes(const D2pcConfig *cfg, size_t *bytes);
 int d2pc_voxel_table_init(const D2pcConfig *cfg, void *d_table, size_t table_bytes, void *stream);
 int d2pc_voxel_enqueue(const D2pcConfig *cfg, double voxel_size, const float *d_xyz,
