@@ -11,6 +11,9 @@ runs in milliseconds and is deterministic, and the spec is our own (DESIGN.md, r
     save_mesh_ply(mesh, "scene")                          # outputs/scene.ply, Open3D's binary layout
 
 Run by ``d2pc_grid_mesh_enqueue``; vertex normals follow Open3D's ``ComputeVertexNormals`` (float64).
+``simplify_mesh`` (row m2, ``d2pc_mesh_simplify_enqueue``) reduces such a mesh by vertex clustering, e.g. for a preview:
+
+    small = simplify_mesh(mesh, voxel_size=0.02)           # contraction="average" or "quadric"
 """
 from __future__ import annotations
 
@@ -102,6 +105,86 @@ def grid_mesh(points, colors, lattice_shape, *, keep=None, max_edge=None, max_an
         if return_device:
             return mesh
         return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in mesh))
+
+
+CONTRACTIONS = ("average", "quadric")
+_SIMPLIFY_ERRORS = ((1, "voxel_size is too small."), (2, "a triangle refers to a vertex that does not exist"),
+                    (4, "the mesh has a non-finite vertex (coordinate, colour or normal)"))
+
+
+def check_voxel_size(voxel_size) -> float:
+    vs = float(voxel_size)
+    if not (math.isfinite(vs) and vs > 0.0):
+        raise ValueError("voxel_size must be a positive finite number")
+    return vs
+
+
+def _device_array(x, dtype, cols, dev):
+    if isinstance(x, torch.Tensor):
+        t = x.to(dev)
+    else:
+        np_dtype = {torch.float32: np.float32, torch.float64: np.float64, torch.int32: np.int32, torch.int64: np.int64}
+        t = torch.from_numpy(np.ascontiguousarray(x, dtype=np_dtype[dtype])).to(dev)
+    if t.dtype != dtype:
+        raise ValueError(f"expected {dtype}, got {t.dtype}")
+    return (t.reshape(-1, cols) if cols else t.reshape(-1)).contiguous()
+
+
+def simplify_mesh(mesh: TriangleMesh, voxel_size: float, *, contraction: str = "average", device=None,
+                  return_device: bool = False) -> TriangleMesh:
+    """Row m2: vertex-clustering simplification (Open3D ``simplify_vertex_clustering``) of a ``TriangleMesh`` -- the
+    NumPy arrays ``grid_mesh`` returns or its CUDA tensors.  Every occupied voxel of size ``voxel_size`` (the ax-2
+    grid on the vertices' bounds) becomes one vertex, ordered by its lowest member vertex; ``contraction`` places it
+    at the members' mean ("average") or at the minimiser of their triangles' plane quadrics when that is well
+    conditioned and inside the voxel ("quadric").  Colours are averaged and normals (when the mesh has them) summed
+    and normalised; triangles are remapped, collapsed and repeated ones dropped.  Raises ValueError for bad
+    arguments, a voxel index of 2^21 or more, a triangle id outside the vertices, and a non-finite vertex."""
+    vs = check_voxel_size(voxel_size)
+    if contraction not in CONTRACTIONS:
+        raise ValueError(f"contraction must be one of {CONTRACTIONS}")
+    nv, nt = len(mesh.vertices), len(mesh.triangles)
+    if nv >= 2 ** 24 or nt >= 2 ** 31:
+        raise ValueError("simplify_mesh takes fewer than 2^24 vertices and 2^31 triangles")
+    lib = _lib.load_library()
+    if not torch.cuda.is_available():
+        raise RuntimeError("image_to_pointcloud_b200 needs a CUDA device (no CPU fallback exists)")
+    if isinstance(mesh.vertices, torch.Tensor):
+        dev = mesh.vertices.device
+    else:
+        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+    with torch.cuda.device(dev):
+        xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
+        rgb = _device_array(mesh.colors, torch.float32, 3, dev)
+        tri = _device_array(mesh.triangles, torch.int32, 3, dev)
+        rows = _device_array(mesh.vertex_rows, torch.int64, 0, dev)
+        nrm = None if mesh.vertex_normals is None else _device_array(mesh.vertex_normals, torch.float64, 3, dev)
+        if len(rgb) != nv or len(rows) != nv or (nrm is not None and len(nrm) != nv):
+            raise ValueError("colors, vertex_rows and vertex_normals must have one row per vertex")
+        nb = C.c_size_t(0)
+        check(lib.d2pc_mesh_simplify_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_simplify_scratch_bytes")
+        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+        oxyz = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+        orgb = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+        orow = torch.empty(nv, dtype=torch.int64, device=dev)
+        onrm = torch.empty((nv, 3), dtype=torch.float64, device=dev) if nrm is not None else None
+        otri = torch.empty((nt, 3), dtype=torch.int32, device=dev)
+        words = torch.zeros(3, dtype=torch.int32, device=dev)   # vertices, triangles, error
+        flags = (_lib.SIMPLIFY_QUADRIC if contraction == "quadric" else 0) | (_lib.SIMPLIFY_NORMALS if nrm is not None else 0)
+
+        def ptr(t):
+            return t.data_ptr() if t is not None and t.numel() > 0 else None
+        check(lib.d2pc_mesh_simplify_enqueue(ptr(xyz), ptr(rgb), ptr(nrm), ptr(rows), nv, ptr(tri), nt, vs, flags,
+                                             scratch.data_ptr(), scratch.numel(), ptr(oxyz), ptr(orgb), ptr(onrm),
+                                             ptr(orow), words.data_ptr(), ptr(otri), words.data_ptr() + 4,
+                                             words.data_ptr() + 8, _stream(dev)),
+              "d2pc_mesh_simplify_enqueue")
+        kv, kt, err = (int(v) for v in words.cpu())
+        if err:
+            raise ValueError("; ".join(msg for bit, msg in _SIMPLIFY_ERRORS if err & bit))
+        out = TriangleMesh(oxyz[:kv], orgb[:kv], otri[:kt], onrm[:kv] if onrm is not None else None, orow[:kv])
+        if return_device:
+            return out
+        return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in out))
 
 
 def lattice_shape(img_h: int, img_w: int, density: str):

@@ -38,6 +38,8 @@
  *   m1 lattice mesh (our own spec; the reference meshes with
  *      Poisson / BPA, :271-308)                                -> d2pc_grid_mesh_enqueue,
  *                                                               d2pc_ply_face_records_enqueue
+ *   m2 mesh simplification by vertex clustering (the reference
+ *      decimates its mesh for the preview, :271-308, 508-535)  -> d2pc_mesh_simplify_enqueue
  */
 #ifndef D2PC_H_
 #define D2PC_H_
@@ -349,6 +351,39 @@ int d2pc_grid_mesh_enqueue(const float *d_xyz, const float *d_rgb, const uint8_t
  * *d_tri_count <= capacity rows in use; d_records 16-byte aligned, capacity * 13 bytes. */
 int d2pc_ply_face_records_enqueue(const int32_t *d_tri, const uint32_t *d_tri_count, uint32_t capacity,
                                   uint8_t *d_records, void *stream);
+
+/* m2 -- simplification of ONE triangle mesh by vertex clustering (Open3D SimplifyVertexClustering; our own rules,
+ * oracle/d2pc_simplify_oracle.py).  Vertices are binned with the ax-2 voxel rule (bmin = the vertices' minimum,
+ * vmin = bmin - vs/2, idx = floor((v - vmin) / vs) in float64, idx < 2^21).  Every occupied cluster becomes one vertex,
+ * ordered by its lowest member vertex id, whose vertex row it takes; its colour is the members' mean, its normal
+ * (with D2PC_SIMPLIFY_NORMALS) the members' normalised sum ((0, 0, 0) for a zero sum), its position the members' mean
+ * or, with D2PC_SIMPLIFY_QUADRIC, the minimiser x = -A^-1 b of the summed plane quadrics of the triangles at its
+ * members (A = sum of area n n^T, b = sum of area d n, once per triangle corner) when det A > 1e-4 trace(A)^3 and x
+ * lies in the cluster's own cell, else the mean.  Triangles are mapped to cluster ids; collapsed ones are dropped,
+ * the rest rotated to start at their smallest id, and only the first of each rotation (by input index) stays, in
+ * input order.
+ *   d_vtx_xyz/rgb     float32 [vertices, 3]; d_vtx_normals float64 [vertices, 3] (with D2PC_SIMPLIFY_NORMALS);
+ *                     d_vtx_row int64 [vertices]; d_tri int32 [triangles, 3]
+ *   d_scratch         d2pc_mesh_simplify_scratch_bytes(vertices, triangles) bytes, 256-byte aligned
+ *   d_out_xyz/rgb     float32 [vertices, 3]; d_out_normals float64 [vertices, 3] (with D2PC_SIMPLIFY_NORMALS);
+ *                     d_out_row int64 [vertices]; d_out_vtx_count uint32 [1]
+ *   d_out_tri         int32 [triangles, 3]; d_out_tri_count uint32 [1]
+ *   d_error           int32 [1]: bit 1 = a cluster index >= 2^21 (voxel_size too small), bit 2 = a triangle id
+ *                     outside [0, vertices), bit 4 = a vertex with a non-finite coordinate, colour or normal; any
+ *                     error leaves both counts 0
+ * Sums are 64-bit fixed point (positions and the quadric scaled to the mesh's extent and total area, colours to
+ * their largest magnitude, normals in two words), so the result repeats bit for bit: colour means are exact for
+ * integral colours, position means are within 2^-38 * extent of the exact means (plus the float32 rounding).
+ * voxel_size finite and > 0; vertices >= 2^24 or triangles >= 2^31 return D2PC_ERR_UNSUPPORTED.  Argument errors
+ * are returned before any launch; the call does not synchronise. */
+enum { D2PC_SIMPLIFY_QUADRIC = 1, D2PC_SIMPLIFY_NORMALS = 2 };
+int d2pc_mesh_simplify_scratch_bytes(uint32_t vertices, uint32_t triangles, size_t *bytes);
+int d2pc_mesh_simplify_enqueue(const float *d_vtx_xyz, const float *d_vtx_rgb, const double *d_vtx_normals,
+                               const int64_t *d_vtx_row, uint32_t vertices, const int32_t *d_tri, uint32_t triangles,
+                               double voxel_size, uint32_t flags, void *d_scratch, size_t scratch_bytes,
+                               float *d_out_xyz, float *d_out_rgb, double *d_out_normals, int64_t *d_out_row,
+                               uint32_t *d_out_vtx_count, int32_t *d_out_tri, uint32_t *d_out_tri_count,
+                               int32_t *d_error, void *stream);
 
 #ifdef __cplusplus
 }
