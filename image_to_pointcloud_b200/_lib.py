@@ -25,6 +25,8 @@ EXPORTS = [
     "d2pc_ply_normal_records_enqueue", "d2pc_normals_scratch_bytes", "d2pc_normals_enqueue",
     "d2pc_grid_mesh_scratch_bytes", "d2pc_grid_mesh_enqueue", "d2pc_ply_face_records_enqueue",
     "d2pc_mesh_simplify_scratch_bytes", "d2pc_mesh_simplify_enqueue",
+    "d2pc_mesh_components_scratch_bytes", "d2pc_mesh_components_enqueue", "d2pc_mesh_filter_scratch_bytes",
+    "d2pc_mesh_filter_enqueue",
     "d2pc_path_create", "d2pc_path_destroy", "d2pc_path_enqueue", "d2pc_path_trace_offset",
 ]
 
@@ -118,6 +120,12 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.d2pc_mesh_simplify_scratch_bytes.argtypes = [C.c_uint32, C.c_uint32, C.POINTER(C.c_size_t)]
     lib.d2pc_mesh_simplify_enqueue.argtypes = [vp, vp, vp, vp, C.c_uint32, vp, C.c_uint32, C.c_double, C.c_uint32, vp,
                                                C.c_size_t, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    lib.d2pc_mesh_components_scratch_bytes.argtypes = [C.c_uint32, C.c_uint32, C.POINTER(C.c_size_t)]
+    lib.d2pc_mesh_components_enqueue.argtypes = [vp, C.c_uint32, vp, C.c_uint32, vp, C.c_size_t, vp, vp, vp, vp, vp,
+                                                 vp]
+    lib.d2pc_mesh_filter_scratch_bytes.argtypes = [C.c_uint32, C.c_uint32, C.POINTER(C.c_size_t)]
+    lib.d2pc_mesh_filter_enqueue.argtypes = [vp, vp, vp, vp, C.c_uint32, vp, C.c_uint32, vp, C.c_uint32, vp,
+                                             C.c_size_t, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.d2pc_path_trace_offset.argtypes = [cfgp, C.POINTER(C.c_size_t)]
     lib.d2pc_path_create.argtypes = [C.POINTER(vp)]
     lib.d2pc_path_destroy.argtypes = [vp]

@@ -28,12 +28,11 @@
 #include <cmath>
 
 #include "d2pc_device.cuh"
+#include "d2pc_scan.cuh"
 
 namespace d2pc {
 
 constexpr int kSimpThreads = 256;
-constexpr int kSimpScanThreads = 1024;
-constexpr int kSimpScanPerThread = 4;
 constexpr int kSimpBits = 21;
 constexpr uint32_t kSimpNone = 0xFFFFFFFFu;
 constexpr unsigned long long kSimpNoKey = 0xFFFFFFFFFFFFFFFFull;
@@ -100,24 +99,6 @@ __device__ __forceinline__ double simp_scale(double x, int k) {
   int ex = 0;
   if (x > 0.0) frexp(x, &ex);
   return ldexp(1.0, k - ex);
-}
-
-// exclusive scan of one value per thread over the CTA; *total = CTA sum
-__device__ __forceinline__ uint32_t simp_excl_scan(uint32_t v, uint32_t *s_warp, uint32_t *total) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  uint32_t incl = v;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    const uint32_t y = __shfl_up_sync(0xffffffffu, incl, d);
-    if (lane >= d) incl += y;
-  }
-  if (lane == 31) s_warp[warp] = incl;
-  __syncthreads();
-  uint32_t woff = 0, t = 0;
-  for (int k = 0; k < nw; ++k) { const uint32_t x = s_warp[k]; if (k < warp) woff += x; t += x; }
-  *total = t;
-  __syncthreads();
-  return woff + incl - v;
 }
 
 __global__ void simp_setup_kernel(SimpArgs a, const float *bounds) {
@@ -211,37 +192,12 @@ __global__ void __launch_bounds__(kSimpThreads) simp_head_kernel(SimpArgs a) {
   if (threadIdx.x == 0) a.vtile[blockIdx.x] = n;
 }
 
-// exclusive scan in place of one tile-count array (one CTA); the total goes to *total
-__global__ void __launch_bounds__(kSimpScanThreads) simp_scan_kernel(uint32_t *arr, uint32_t n, uint32_t *total_out) {
-  __shared__ uint32_t s_warp[32];
-  __shared__ uint32_t s_carry;
-  if (threadIdx.x == 0) s_carry = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < n; base += kSimpScanThreads * kSimpScanPerThread) {
-    const uint32_t i0 = base + threadIdx.x * kSimpScanPerThread;
-    uint32_t v[kSimpScanPerThread], sum = 0;
-#pragma unroll
-    for (int k = 0; k < kSimpScanPerThread; ++k) { v[k] = i0 + k < n ? arr[i0 + k] : 0u; sum += v[k]; }
-    uint32_t total;
-    uint32_t ex = s_carry + simp_excl_scan(sum, s_warp, &total);
-#pragma unroll
-    for (int k = 0; k < kSimpScanPerThread; ++k) {
-      if (i0 + k < n) arr[i0 + k] = ex;
-      ex += v[k];
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) s_carry += total;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) *total_out = s_carry;
-}
-
 __global__ void __launch_bounds__(kSimpThreads) simp_assign_kernel(SimpArgs a) {
   __shared__ uint32_t s_warp[kSimpThreads / 32];
   const uint32_t i = blockIdx.x * kSimpThreads + threadIdx.x;
   const bool head = simp_is_head(a, i);
   uint32_t total;
-  const uint32_t id = a.vtile[blockIdx.x] + simp_excl_scan(head ? 1u : 0u, s_warp, &total);
+  const uint32_t id = a.vtile[blockIdx.x] + tile_excl_scan(head ? 1u : 0u, s_warp, &total);
   if (!head) return;
   const uint32_t s = a.vslot[i];
   a.slot_cid[s] = id;
@@ -419,7 +375,7 @@ __global__ void __launch_bounds__(kSimpThreads) simp_tri_write_kernel(SimpArgs a
   const uint32_t t = blockIdx.x * kSimpThreads + threadIdx.x;
   const bool keep = simp_tri_kept(a, t);
   uint32_t total;
-  const uint32_t j = a.ttile[blockIdx.x] + simp_excl_scan(keep ? 1u : 0u, s_warp, &total);
+  const uint32_t j = a.ttile[blockIdx.x] + tile_excl_scan(keep ? 1u : 0u, s_warp, &total);
   if (!keep) return;
 #pragma unroll
   for (int k = 0; k < 3; ++k) a.otri[3 * (size_t)j + k] = (int32_t)a.canon[3 * (size_t)t + k];
@@ -632,7 +588,7 @@ extern "C" int d2pc_mesh_simplify_enqueue(const float *d_vtx_xyz, const float *d
   D2PC_CHECK_LAUNCH();
   simp_head_kernel<<<L.vtiles, kSimpThreads, 0, st>>>(a);
   D2PC_CHECK_LAUNCH();
-  simp_scan_kernel<<<1, kSimpScanThreads, 0, st>>>(a.vtile, L.vtiles, &a.hdr->n_clusters);
+  tile_scan_kernel<<<1, kTileScanThreads, 0, st>>>(a.vtile, L.vtiles, &a.hdr->n_clusters);
   D2PC_CHECK_LAUNCH();
   simp_assign_kernel<<<L.vtiles, kSimpThreads, 0, st>>>(a);
   D2PC_CHECK_LAUNCH();
@@ -652,7 +608,7 @@ extern "C" int d2pc_mesh_simplify_enqueue(const float *d_vtx_xyz, const float *d
     D2PC_CHECK_LAUNCH();
     simp_tri_flag_kernel<<<L.ttiles, kSimpThreads, 0, st>>>(a);
     D2PC_CHECK_LAUNCH();
-    simp_scan_kernel<<<1, kSimpScanThreads, 0, st>>>(a.ttile, L.ttiles, &a.hdr->n_tri);
+    tile_scan_kernel<<<1, kTileScanThreads, 0, st>>>(a.ttile, L.ttiles, &a.hdr->n_tri);
     D2PC_CHECK_LAUNCH();
     simp_tri_write_kernel<<<L.ttiles, kSimpThreads, 0, st>>>(a);
     D2PC_CHECK_LAUNCH();

@@ -14,6 +14,12 @@ Run by ``d2pc_grid_mesh_enqueue``; vertex normals follow Open3D's ``ComputeVerte
 ``simplify_mesh`` (row m2, ``d2pc_mesh_simplify_enqueue``) reduces such a mesh by vertex clustering, e.g. for a preview:
 
     small = simplify_mesh(mesh, voxel_size=0.02)           # contraction="average" or "quadric"
+
+Row m3 (``d2pc_mesh_components_enqueue``, ``d2pc_mesh_filter_enqueue``) finds the edge-connected components of a
+mesh (Open3D ``cluster_connected_triangles``) and removes triangles by a mask, e.g. the small islands a depth cut
+leaves in front of the surface:
+
+    clean = remove_small_components(mesh, min_triangles=10)
 """
 from __future__ import annotations
 
@@ -187,6 +193,153 @@ def simplify_mesh(mesh: TriangleMesh, voxel_size: float, *, contraction: str = "
         return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in out))
 
 
+_COMPONENT_ERRORS = ((1, "a triangle refers to a vertex that does not exist"),
+                     (2, "the mesh has a non-finite vertex coordinate"))
+_COMPONENT_MAX_TRIANGLES = 2 ** 25
+
+
+def _mesh_device(mesh, device):
+    lib = _lib.load_library()
+    if not torch.cuda.is_available():
+        raise RuntimeError("image_to_pointcloud_b200 needs a CUDA device (no CPU fallback exists)")
+    if len(mesh.triangles) > _COMPONENT_MAX_TRIANGLES or len(mesh.vertices) > 2 ** 31:
+        raise ValueError("meshes of at most 2^25 triangles and 2^31 vertices are supported")
+    if isinstance(mesh.vertices, torch.Tensor):
+        return lib, mesh.vertices.device
+    return lib, torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+
+
+def _raise_component_errors(err: int, where: str) -> None:
+    if err & ~3:
+        raise RuntimeError(f"{where}: a device loop exhausted its bound (error word {err})")
+    if err:
+        raise ValueError("; ".join(msg for bit, msg in _COMPONENT_ERRORS if err & bit))
+
+
+def _ptr(t):
+    return t.data_ptr() if t is not None and t.numel() > 0 else None
+
+
+def cluster_connected_triangles(mesh: TriangleMesh, *, device=None, return_device: bool = False):
+    """Row m3: Open3D's ``cluster_connected_triangles`` of a ``TriangleMesh`` (NumPy arrays or CUDA tensors):
+    ``(triangle_clusters int32 [T], cluster_n_triangles int64 [K], cluster_area float64 [K])``.  Two triangles are
+    connected when they share an edge; clusters are numbered by their lowest triangle.  Areas are Open3D's triangle
+    areas summed in 64-bit fixed point (DESIGN.md, row m3), so they repeat bit for bit.  Raises ValueError for a
+    triangle id outside the vertices and a non-finite vertex coordinate."""
+    lib, dev = _mesh_device(mesh, device)
+    nv, nt = len(mesh.vertices), len(mesh.triangles)
+    with torch.cuda.device(dev):
+        xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
+        tri = _device_array(mesh.triangles, torch.int32, 3, dev)
+        nb = C.c_size_t(0)
+        check(lib.d2pc_mesh_components_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_components_scratch_bytes")
+        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+        labels = torch.empty(nt, dtype=torch.int32, device=dev)
+        n = torch.empty(nt, dtype=torch.int64, device=dev)
+        area = torch.empty(nt, dtype=torch.float64, device=dev)
+        words = torch.zeros(2, dtype=torch.int32, device=dev)   # K, error
+        check(lib.d2pc_mesh_components_enqueue(_ptr(xyz), nv, _ptr(tri), nt, scratch.data_ptr(), scratch.numel(),
+                                               _ptr(labels), _ptr(n), _ptr(area), words.data_ptr(),
+                                               words.data_ptr() + 4, _stream(dev)),
+              "d2pc_mesh_components_enqueue")
+        k, err = (int(v) for v in words.cpu())
+        _raise_component_errors(err, "cluster_connected_triangles")
+        out = (labels, n[:k], area[:k])
+        if return_device:
+            return out
+        return tuple(t.cpu().numpy() for t in out)
+
+
+def remove_triangles_by_mask(mesh: TriangleMesh, mask, *, remove_unreferenced: bool = True, device=None,
+                             return_device: bool = False) -> TriangleMesh:
+    """Row m3: Open3D's ``remove_triangles_by_mask`` (``mask`` bool [T], True: the triangle goes), then with
+    ``remove_unreferenced`` its ``remove_unreferenced_vertices``.  Kept triangles and vertices keep their order;
+    colours, normals and vertex rows are carried unchanged (normals are not recomputed).  Raises ValueError for a
+    triangle id outside the vertices and a non-finite vertex coordinate."""
+    lib, dev = _mesh_device(mesh, device)
+    nv, nt = len(mesh.vertices), len(mesh.triangles)
+    with torch.cuda.device(dev):
+        m = mask if isinstance(mask, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(mask))
+        m = m.to(dev).reshape(-1)
+        if m.numel() != nt:
+            raise ValueError("the mask must have one entry per triangle")
+        keep = (m == 0).to(torch.uint8).contiguous()
+        return _filter(lib, dev, mesh, keep, remove_unreferenced, return_device)
+
+
+def _filter(lib, dev, mesh, keep, remove_unreferenced, return_device):
+    nv, nt = len(mesh.vertices), len(mesh.triangles)
+    xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
+    rgb = _device_array(mesh.colors, torch.float32, 3, dev)
+    tri = _device_array(mesh.triangles, torch.int32, 3, dev)
+    rows = _device_array(mesh.vertex_rows, torch.int64, 0, dev)
+    nrm = None if mesh.vertex_normals is None else _device_array(mesh.vertex_normals, torch.float64, 3, dev)
+    if len(rgb) != nv or len(rows) != nv or (nrm is not None and len(nrm) != nv):
+        raise ValueError("colors, vertex_rows and vertex_normals must have one row per vertex")
+    nb = C.c_size_t(0)
+    check(lib.d2pc_mesh_filter_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_filter_scratch_bytes")
+    scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+    oxyz = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+    orgb = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+    orow = torch.empty(nv, dtype=torch.int64, device=dev)
+    onrm = torch.empty((nv, 3), dtype=torch.float64, device=dev) if nrm is not None else None
+    otri = torch.empty((nt, 3), dtype=torch.int32, device=dev)
+    words = torch.zeros(3, dtype=torch.int32, device=dev)   # vertices, triangles, error
+    flags = (_lib.MESH_REMOVE_UNREFERENCED if remove_unreferenced else 0) | (_lib.MESH_NORMALS if nrm is not None else 0)
+    check(lib.d2pc_mesh_filter_enqueue(_ptr(xyz), _ptr(rgb), _ptr(nrm), _ptr(rows), nv, _ptr(tri), nt, _ptr(keep),
+                                       flags, scratch.data_ptr(), scratch.numel(), _ptr(oxyz), _ptr(orgb), _ptr(onrm),
+                                       _ptr(orow), words.data_ptr(), _ptr(otri), words.data_ptr() + 4,
+                                       words.data_ptr() + 8, _stream(dev)),
+          "d2pc_mesh_filter_enqueue")
+    kv, kt, err = (int(v) for v in words.cpu())
+    _raise_component_errors(err, "remove_triangles_by_mask")
+    out = TriangleMesh(oxyz[:kv], orgb[:kv], otri[:kt], onrm[:kv] if onrm is not None else None, orow[:kv])
+    if return_device:
+        return out
+    return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in out))
+
+
+def check_min_triangles(min_triangles) -> int:
+    n = int(min_triangles)
+    if n != min_triangles or n < 1:
+        raise ValueError("min_triangles must be an integer >= 1")
+    return n
+
+
+def _small_components(mesh, min_triangles, min_area, remove_unreferenced, device, return_device):
+    """(cleaned mesh, K, removed triangles)."""
+    if min_triangles is None and min_area is None:
+        raise ValueError("give min_triangles, min_area or both")
+    if min_triangles is not None:
+        min_triangles = check_min_triangles(min_triangles)
+    if min_area is not None:
+        min_area = float(min_area)
+        if math.isnan(min_area):
+            raise ValueError("min_area must be a number")
+    lib, dev = _mesh_device(mesh, device)
+    with torch.cuda.device(dev):
+        labels, n, area = cluster_connected_triangles(mesh, device=dev, return_device=True)
+        lab = labels.to(torch.int64)
+        remove = torch.zeros(labels.numel(), dtype=torch.bool, device=dev)
+        if min_triangles is not None:
+            remove |= n[lab] < min_triangles
+        if min_area is not None:
+            remove |= area[lab] < min_area
+        keep = (~remove).to(torch.uint8)
+        out = _filter(lib, dev, mesh, keep, remove_unreferenced, return_device)
+        return out, int(n.numel()), len(mesh.triangles) - len(out.triangles)
+
+
+def remove_small_components(mesh: TriangleMesh, *, min_triangles: Optional[int] = None,
+                            min_area: Optional[float] = None, device=None, return_device: bool = False) -> TriangleMesh:
+    """Row m3: removes every connected component (``cluster_connected_triangles``) with fewer than ``min_triangles``
+    triangles or less area than ``min_area``, then the vertices no kept triangle uses -- Open3D's
+    ``remove_triangles_by_mask(cluster_n_triangles[triangle_clusters] < N)`` and ``remove_unreferenced_vertices``,
+    entirely on the device.  Raises ValueError for bad arguments, a triangle id outside the vertices and a non-finite
+    vertex coordinate."""
+    return _small_components(mesh, min_triangles, min_area, True, device, return_device)[0]
+
+
 def lattice_shape(img_h: int, img_w: int, density: str):
     """(R, C) of the emit lattice: ceil(H / step) x ceil(W / step)."""
     s = DENSITY_STEP[density]
@@ -210,16 +363,20 @@ def depth_to_mesh(image: np.ndarray, depth: np.ndarray, density: str = "medium",
                   depth_scale: float = 10.0, smooth: bool = False, smooth_ksize: int = 5, fov: Optional[float] = None,
                   *, z_range=None, refine: bool = False, nb_neighbors: int = 20, std_ratio: float = 2.0,
                   max_edge=None, max_angle: float = 85.0, remove_unreferenced: bool = True,
-                  compute_normals: bool = True, device=None, return_device: bool = False) -> TriangleMesh:
+                  compute_normals: bool = True, min_component_triangles: Optional[int] = None, device=None,
+                  return_device: bool = False) -> TriangleMesh:
     """Mesh of one (image, depth) pair in one device-resident pass: the unmasked emit of ``depth_to_point_cloud``
     (same positional arguments), ``z_range`` as a mask on the lattice (the float32 rule of the depth-range mask),
     with ``refine`` statistical outlier removal of the remaining rows (``nb_neighbors``, ``std_ratio``), then
     ``grid_mesh``.  The vertices are the points ``depth_to_point_cloud(..., z_range=z_range)`` followed by
-    ``refine_point_cloud`` would keep (those a kept triangle uses, with ``remove_unreferenced``)."""
+    ``refine_point_cloud`` would keep (those a kept triangle uses, with ``remove_unreferenced``).  With
+    ``min_component_triangles`` the components of fewer triangles are removed (``remove_small_components``)."""
     DENSITY_STEP[density]  # KeyError first, like the reference
     if z_range is not None and len(z_range) != 2:
         raise ValueError("z_range must be (z_min, z_max)")
     _cos2(max_angle), _max_edge(max_edge)   # argument errors before any device work
+    if min_component_triangles is not None:
+        check_min_triangles(min_component_triangles)
     img_h, img_w = image.shape[:2]
     dep_h, dep_w = depth.shape[:2]
     check_depth_dtype(depth, int(img_h), int(img_w))
@@ -240,6 +397,11 @@ def depth_to_mesh(image: np.ndarray, depth: np.ndarray, density: str = "medium",
             keep = ((z >= float(np.float32(z_range[0]))) & (z <= float(np.float32(z_range[1])))).to(torch.uint8)
         if refine:
             keep = refined_keep(xyz, keep, nb_neighbors, std_ratio)
-        return grid_mesh(xyz, rgb, lattice_shape(img_h, img_w, density), keep=keep, max_edge=max_edge,
+        if min_component_triangles is None:
+            return grid_mesh(xyz, rgb, lattice_shape(img_h, img_w, density), keep=keep, max_edge=max_edge,
+                             max_angle=max_angle, remove_unreferenced=remove_unreferenced,
+                             compute_normals=compute_normals, return_device=return_device)
+        mesh = grid_mesh(xyz, rgb, lattice_shape(img_h, img_w, density), keep=keep, max_edge=max_edge,
                          max_angle=max_angle, remove_unreferenced=remove_unreferenced,
-                         compute_normals=compute_normals, return_device=return_device)
+                         compute_normals=compute_normals, return_device=True)
+        return _small_components(mesh, min_component_triangles, None, remove_unreferenced, dev, return_device)[0]

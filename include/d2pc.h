@@ -385,6 +385,52 @@ int d2pc_mesh_simplify_enqueue(const float *d_vtx_xyz, const float *d_vtx_rgb, c
                                uint32_t *d_out_vtx_count, int32_t *d_out_tri, uint32_t *d_out_tri_count,
                                int32_t *d_error, void *stream);
 
+/* m3 -- connected components of ONE triangle mesh (Open3D ClusterConnectedTriangles; our restatement,
+ * oracle/d2pc_components_oracle.py).  Two triangles are connected when they share an edge, an unordered vertex pair
+ * (sharing only a vertex does not connect; a non-manifold edge connects every triangle on it; a degenerate triangle
+ * (a, a, b) has the edges {a,a}, {a,b}, {a,b}).  Clusters are numbered in ascending order of their lowest triangle.
+ * The area of a triangle is Open3D's 0.5 |(p0 - p1) x (p0 - p2)| in float64 (Eigen's component order, the norm summed
+ * left to right); the area of a cluster is sum_t rint(a_t s) / s in 64-bit fixed point with s = 2^(62 - e_a - e_T),
+ * max_t a_t < 2^e_a (frexp; e_a = 0 when every area is 0) and T <= 2^e_T, the integer sum rounded once to float64.
+ *   d_vtx_xyz            float32 [vertices, 3]; d_tri int32 [triangles, 3]
+ *   d_scratch            d2pc_mesh_components_scratch_bytes(vertices, triangles) bytes, 256-byte aligned
+ *   d_out_tri_cluster    int32 [triangles]: cluster of every triangle
+ *   d_out_cluster_n      int64 [triangles], the first K in use: triangles of every cluster
+ *   d_out_cluster_area   float64 [triangles], the first K in use: area of every cluster
+ *   d_out_cluster_count  uint32 [1]: K (0 on an error)
+ *   d_error              int32 [1]: bit 1 = a triangle id outside [0, vertices), bit 2 = a vertex with a non-finite
+ *                        coordinate, bit 4 = a loop bound was exhausted (an internal failure, never expected)
+ * triangles <= 2^25 (twice the 2 * 2159 * 3839 triangles of a 4K lattice mesh) and vertices <= 2^31, else
+ * D2PC_ERR_UNSUPPORTED.  No floating-point atomics: the result repeats bit for bit.  Argument errors are returned
+ * before any launch; the call does not synchronise. */
+int d2pc_mesh_components_scratch_bytes(uint32_t vertices, uint32_t triangles, size_t *bytes);
+int d2pc_mesh_components_enqueue(const float *d_vtx_xyz, uint32_t vertices, const int32_t *d_tri, uint32_t triangles,
+                                 void *d_scratch, size_t scratch_bytes, int32_t *d_out_tri_cluster,
+                                 int64_t *d_out_cluster_n, double *d_out_cluster_area, uint32_t *d_out_cluster_count,
+                                 int32_t *d_error, void *stream);
+
+/* m3 -- removal of triangles by a mask (Open3D RemoveTrianglesByMask, then with D2PC_MESH_REMOVE_UNREFERENCED
+ * RemoveUnreferencedVertices).  Triangle t stays when d_tri_keep[t] != 0; kept triangles keep their input order.
+ * Vertices stay in input order (with D2PC_MESH_REMOVE_UNREFERENCED only those a kept triangle uses), their colour,
+ * row and (with D2PC_MESH_NORMALS) normal carried unchanged, and the kept triangles are remapped to the new ids.
+ *   d_vtx_xyz/rgb        float32 [vertices, 3]; d_vtx_normals float64 [vertices, 3] (with D2PC_MESH_NORMALS);
+ *                        d_vtx_row int64 [vertices]; d_tri int32 [triangles, 3]; d_tri_keep uint8 [triangles]
+ *   d_scratch            d2pc_mesh_filter_scratch_bytes(vertices, triangles) bytes, 256-byte aligned
+ *   d_out_xyz/rgb        float32 [vertices, 3]; d_out_normals float64 [vertices, 3] (with D2PC_MESH_NORMALS);
+ *                        d_out_row int64 [vertices]; d_out_vtx_count uint32 [1]
+ *   d_out_tri            int32 [triangles, 3]; d_out_tri_count uint32 [1]
+ *   d_error              int32 [1]: bit 1 = a triangle id outside [0, vertices), bit 2 = a vertex with a non-finite
+ *                        coordinate; any error leaves both counts 0
+ * The size limits are those of d2pc_mesh_components_enqueue.  Argument errors are returned before any launch; the
+ * call does not synchronise. */
+int d2pc_mesh_filter_scratch_bytes(uint32_t vertices, uint32_t triangles, size_t *bytes);
+int d2pc_mesh_filter_enqueue(const float *d_vtx_xyz, const float *d_vtx_rgb, const double *d_vtx_normals,
+                             const int64_t *d_vtx_row, uint32_t vertices, const int32_t *d_tri, uint32_t triangles,
+                             const uint8_t *d_tri_keep, uint32_t flags, void *d_scratch, size_t scratch_bytes,
+                             float *d_out_xyz, float *d_out_rgb, double *d_out_normals, int64_t *d_out_row,
+                             uint32_t *d_out_vtx_count, int32_t *d_out_tri, uint32_t *d_out_tri_count,
+                             int32_t *d_error, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
