@@ -11,8 +11,9 @@ from .api import create_depth_preview, depth_preview_bgr, depth_to_point_cloud, 
 from .engine import DENSITY_STEP, BatchStream, EmitResult, FrameEngine, reference_intrinsics, shard_frames
 from .hostpipe import HostFramePipeline, MultiGpuPipeline
 from ._lib import D2pcConfig, D2pcError, D2pcFrameParams, load_library
-from .mesh import (TriangleMesh, cluster_connected_triangles, depth_to_mesh, grid_mesh, remove_small_components,
-                   remove_triangles_by_mask, simplify_mesh)
+from .mesh import (TriangleMesh, cluster_connected_triangles, compute_vertex_normals, depth_to_mesh,
+                   filter_smooth_laplacian, filter_smooth_simple, filter_smooth_taubin, grid_mesh,
+                   remove_small_components, remove_triangles_by_mask, simplify_mesh)
 from .normals import estimate_normals
 from .pipeline import point_cloud_stage
 from .refine import refine_point_cloud, statistical_outlier_removal
@@ -27,6 +28,7 @@ __all__ = [
     "save_ply", "save_point_cloud", "refine_point_cloud", "statistical_outlier_removal", "point_cloud_stage",
     "estimate_normals", "grid_mesh", "depth_to_mesh", "TriangleMesh", "ply_face_records", "mesh_ply_bytes",
     "save_mesh_ply", "simplify_mesh", "cluster_connected_triangles", "remove_triangles_by_mask",
-    "remove_small_components",
+    "remove_small_components", "filter_smooth_simple", "filter_smooth_laplacian", "filter_smooth_taubin",
+    "compute_vertex_normals",
 ]
 __version__ = "0.1.0"

@@ -20,6 +20,12 @@ mesh (Open3D ``cluster_connected_triangles``) and removes triangles by a mask, e
 leaves in front of the surface:
 
     clean = remove_small_components(mesh, min_triangles=10)
+
+Row m4 (``d2pc_mesh_smooth_enqueue``, ``d2pc_mesh_vertex_normals_enqueue``) smooths a mesh (Open3D
+``filter_smooth_simple`` / ``filter_smooth_laplacian`` / ``filter_smooth_taubin``) and recomputes the vertex normals of
+any mesh, e.g. to take the terraces of a monocular depth map out of the lattice mesh:
+
+    smooth = compute_vertex_normals(filter_smooth_taubin(mesh, 10, scope="vertex"))
 """
 from __future__ import annotations
 
@@ -338,6 +344,124 @@ def remove_small_components(mesh: TriangleMesh, *, min_triangles: Optional[int] 
     entirely on the device.  Raises ValueError for bad arguments, a triangle id outside the vertices and a non-finite
     vertex coordinate."""
     return _small_components(mesh, min_triangles, min_area, True, device, return_device)[0]
+
+
+SMOOTH_SCOPES = {"all": _lib.SMOOTH_VERTEX | _lib.SMOOTH_NORMAL | _lib.SMOOTH_COLOR, "vertex": _lib.SMOOTH_VERTEX,
+                 "normal": _lib.SMOOTH_NORMAL, "color": _lib.SMOOTH_COLOR}
+_SMOOTH_ERRORS = ((1, "a triangle refers to a vertex that does not exist"),
+                  (2, "the mesh has a non-finite vertex coordinate (or colour / normal in the scope)"))
+
+
+def check_iterations(number_of_iterations) -> int:
+    n = int(number_of_iterations)
+    if n != number_of_iterations or not 0 <= n < 2 ** 31:
+        raise ValueError("number_of_iterations must be an integer >= 0")
+    return n
+
+
+def _finite(name, x) -> float:
+    x = float(x)
+    if not math.isfinite(x):
+        raise ValueError(f"{name} must be a finite number")
+    return x
+
+
+def _host_or_device(out, return_device):
+    if return_device:
+        return out
+    return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in out))
+
+
+def _smooth(mesh, method, iterations, lambda_filter, mu, scope, device, return_device):
+    n = check_iterations(iterations)
+    lam, mu = _finite("lambda_filter", lambda_filter), _finite("mu", mu)
+    if scope not in SMOOTH_SCOPES:
+        raise ValueError(f"scope must be one of {tuple(SMOOTH_SCOPES)}")
+    lib, dev = _mesh_device(mesh, device)
+    nv, nt = len(mesh.vertices), len(mesh.triangles)
+    with torch.cuda.device(dev):
+        xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
+        rgb = _device_array(mesh.colors, torch.float32, 3, dev)
+        tri = _device_array(mesh.triangles, torch.int32, 3, dev)
+        rows = _device_array(mesh.vertex_rows, torch.int64, 0, dev)
+        nrm = None if mesh.vertex_normals is None else _device_array(mesh.vertex_normals, torch.float64, 3, dev)
+        if len(rgb) != nv or len(rows) != nv or (nrm is not None and len(nrm) != nv):
+            raise ValueError("colors, vertex_rows and vertex_normals must have one row per vertex")
+        nb = C.c_size_t(0)
+        check(lib.d2pc_mesh_smooth_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_smooth_scratch_bytes")
+        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+        oxyz = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+        orgb = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+        onrm = torch.empty((nv, 3), dtype=torch.float64, device=dev) if nrm is not None else None
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+        check(lib.d2pc_mesh_smooth_enqueue(_ptr(xyz), _ptr(rgb), _ptr(nrm), nv, _ptr(tri), nt, method, n, lam, mu,
+                                           SMOOTH_SCOPES[scope], scratch.data_ptr(), scratch.numel(), _ptr(oxyz),
+                                           _ptr(orgb), _ptr(onrm), err.data_ptr(), _stream(dev)),
+              "d2pc_mesh_smooth_enqueue")
+        e = int(err.cpu())
+        _raise_smooth_errors(e, "mesh smoothing")
+        return _host_or_device(TriangleMesh(oxyz, orgb, tri, onrm, rows), return_device)
+
+
+def _raise_smooth_errors(err: int, where: str) -> None:
+    if err & ~3:
+        raise RuntimeError(f"{where}: a device loop exhausted its bound (error word {err})")
+    if err:
+        raise ValueError("; ".join(msg for bit, msg in _SMOOTH_ERRORS if err & bit))
+
+
+def filter_smooth_simple(mesh: TriangleMesh, number_of_iterations: int = 1, *, scope: str = "all", device=None,
+                         return_device: bool = False) -> TriangleMesh:
+    """Row m4: Open3D's ``filter_smooth_simple`` of a ``TriangleMesh`` (NumPy arrays or CUDA tensors): every pass
+    moves each vertex to the mean of itself and its neighbours (Open3D's adjacency sets, visited in ascending id),
+    in float64, rounded to float32 once at the end.  ``scope`` ("all", "vertex", "normal", "color") picks the fields
+    filtered (normals only when the mesh has them; they are not renormalised); triangles and vertex rows are kept.
+    Raises ValueError for bad arguments, a triangle id outside the vertices and a non-finite value."""
+    return _smooth(mesh, _lib.SMOOTH_SIMPLE, number_of_iterations, 0.5, -0.53, scope, device, return_device)
+
+
+def filter_smooth_laplacian(mesh: TriangleMesh, number_of_iterations: int = 1, lambda_filter: float = 0.5, *,
+                            scope: str = "all", device=None, return_device: bool = False) -> TriangleMesh:
+    """Row m4: Open3D's ``filter_smooth_laplacian``: every pass moves each vertex by ``lambda_filter`` towards the mean
+    of its neighbours weighted by 1 / (distance + 1e-12); colours and normals take the same weights.  A vertex
+    without neighbours stays as it is (Open3D writes NaN).  Otherwise as ``filter_smooth_simple``."""
+    return _smooth(mesh, _lib.SMOOTH_LAPLACIAN, number_of_iterations, lambda_filter, -0.53, scope, device,
+                   return_device)
+
+
+def filter_smooth_taubin(mesh: TriangleMesh, number_of_iterations: int = 1, lambda_filter: float = 0.5,
+                         mu: float = -0.53, *, scope: str = "all", device=None,
+                         return_device: bool = False) -> TriangleMesh:
+    """Row m4: Open3D's ``filter_smooth_taubin``: every iteration is a Laplacian pass with ``lambda_filter``, then one
+    with ``mu``, which smooths without the shrinking of the plain Laplacian.  Otherwise as
+    ``filter_smooth_laplacian``."""
+    return _smooth(mesh, _lib.SMOOTH_TAUBIN, number_of_iterations, lambda_filter, mu, scope, device, return_device)
+
+
+def compute_vertex_normals(mesh: TriangleMesh, *, device=None, return_device: bool = False) -> TriangleMesh:
+    """Row m4: the mesh with its ``vertex_normals`` replaced by Open3D's ``compute_vertex_normals``, m1's rule: the
+    unnormalised normals of every vertex's triangles summed in ascending triangle order and normalised ((0, 0, 1) for
+    a zero sum), float64 -- bit for bit the normals ``grid_mesh`` computes.  Raises ValueError for a triangle id
+    outside the vertices and a non-finite vertex coordinate."""
+    lib, dev = _mesh_device(mesh, device)
+    nv, nt = len(mesh.vertices), len(mesh.triangles)
+    with torch.cuda.device(dev):
+        xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
+        rgb = _device_array(mesh.colors, torch.float32, 3, dev)
+        tri = _device_array(mesh.triangles, torch.int32, 3, dev)
+        rows = _device_array(mesh.vertex_rows, torch.int64, 0, dev)
+        if len(rgb) != nv or len(rows) != nv:
+            raise ValueError("colors and vertex_rows must have one row per vertex")
+        nb = C.c_size_t(0)
+        check(lib.d2pc_mesh_vertex_normals_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_vertex_normals_scratch_bytes")
+        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+        onrm = torch.empty((nv, 3), dtype=torch.float64, device=dev)
+        err = torch.zeros(1, dtype=torch.int32, device=dev)
+        check(lib.d2pc_mesh_vertex_normals_enqueue(_ptr(xyz), nv, _ptr(tri), nt, scratch.data_ptr(), scratch.numel(),
+                                                   _ptr(onrm), err.data_ptr(), _stream(dev)),
+              "d2pc_mesh_vertex_normals_enqueue")
+        _raise_smooth_errors(int(err.cpu()), "compute_vertex_normals")
+        return _host_or_device(TriangleMesh(xyz, rgb, tri, onrm, rows), return_device)
 
 
 def lattice_shape(img_h: int, img_w: int, density: str):

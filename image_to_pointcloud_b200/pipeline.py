@@ -6,6 +6,7 @@
     [-> estimate_normals, the mesh builder's first step (:271-308), with normals=True]
     [-> grid_mesh of the refined lattice rows, the mesh PLY (row m1), with mesh=True]
     [-> remove_small_components of that mesh (row m3), with mesh_min_triangles]
+    [-> filter_smooth_taubin and compute_vertex_normals of that mesh (row m4), with mesh_smooth_iterations]
     [-> simplify_mesh of that mesh, the preview mesh PLY (row m2), with mesh_preview_voxel]
 
 Called as separate drop-ins, those steps move the cloud across PCIe five times (down after the stage, up
@@ -27,8 +28,8 @@ from . import _lib, writers
 from ._lib import check
 from .api import _engine_for, _image_channels, _to_host, bounds_dict, check_depth_dtype
 from .engine import DENSITY_STEP
-from .mesh import (_cos2, _max_edge, _small_components, check_min_triangles, check_voxel_size, grid_mesh,
-                   lattice_shape, simplify_mesh)
+from .mesh import (_cos2, _max_edge, _small_components, check_iterations, check_min_triangles, check_voxel_size,
+                   compute_vertex_normals, filter_smooth_taubin, grid_mesh, lattice_shape, simplify_mesh)
 from .normals import estimate_normals
 from .refine import statistical_outlier_removal
 
@@ -40,7 +41,7 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
                       max_preview: int = writers.MAX_PREVIEW, return_arrays: bool = True, normals: bool = False,
                       normals_knn: int = 30, mesh: bool = False, mesh_max_angle: float = 85.0, mesh_max_edge=None,
                       mesh_preview_voxel: Optional[float] = None, mesh_min_triangles: Optional[int] = None,
-                      device=None) -> dict:
+                      mesh_smooth_iterations: Optional[int] = None, device=None) -> dict:
     """Returns a dict with ``points`` / ``colors`` (host float32 [M,3], if ``return_arrays``), ``point_count``,
     ``preview_points`` / ``preview_colors`` (nested lists as app.py:505-506), ``bounds`` (app.py:393-400),
     and either ``filepath`` (``filename`` given: the file the reference's writer would have put into
@@ -51,8 +52,11 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
     ``mesh_vertex_count``, ``mesh_triangle_count`` and either ``mesh_filepath`` (outputs/<filename>_mesh.ply) or
     ``mesh_file_bytes``.  With ``mesh_min_triangles`` (needs ``mesh``) the components of fewer triangles are removed
     from that mesh before it is written (``remove_small_components``): ``mesh_component_count`` (before the removal)
-    and ``mesh_removed_triangle_count``, the counts above describing the cleaned mesh.  With ``mesh_preview_voxel``
-    (needs ``mesh``) that mesh is also simplified for a preview (``simplify_mesh(mesh, mesh_preview_voxel)``, average
+    and ``mesh_removed_triangle_count``, the counts above describing the cleaned mesh.  With
+    ``mesh_smooth_iterations`` (needs ``mesh``) that mesh is then smoothed (``filter_smooth_taubin(mesh, N, 0.5, -0.53,
+    scope="vertex")``) and its vertex normals recomputed (``compute_vertex_normals``) before it is written; 0 keeps
+    the positions and still recomputes the normals.  With ``mesh_preview_voxel`` (needs ``mesh``) that (cleaned,
+    smoothed) mesh is also simplified for a preview (``simplify_mesh(mesh, mesh_preview_voxel)``, average
     contraction): ``mesh_preview_vertex_count``,
     ``mesh_preview_triangle_count`` and either ``mesh_preview_filepath`` (outputs/<filename>_mesh_preview.ply) or
     ``mesh_preview_file_bytes``."""
@@ -67,6 +71,10 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
         if not mesh:
             raise ValueError("mesh_min_triangles needs mesh=True")
         check_min_triangles(mesh_min_triangles)
+    if mesh_smooth_iterations is not None:
+        if not mesh:
+            raise ValueError("mesh_smooth_iterations needs mesh=True")
+        check_iterations(mesh_smooth_iterations)
     lib = _lib.load_library()
     img_h, img_w = image.shape[:2]
     dep_h, dep_w = depth.shape[:2]
@@ -134,6 +142,9 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
             if mesh_min_triangles is not None:
                 msh, out["mesh_component_count"], out["mesh_removed_triangle_count"] = _small_components(
                     msh, mesh_min_triangles, None, True, dev, True)
+            if mesh_smooth_iterations is not None:
+                msh = filter_smooth_taubin(msh, mesh_smooth_iterations, 0.5, -0.53, scope="vertex", return_device=True)
+                msh = compute_vertex_normals(msh, return_device=True)
             out["mesh_vertex_count"], out["mesh_triangle_count"] = len(msh.vertices), len(msh.triangles)
             if filename is not None:
                 out["mesh_filepath"] = writers.save_mesh_ply(msh, f"{filename}_mesh")

@@ -431,6 +431,49 @@ int d2pc_mesh_filter_enqueue(const float *d_vtx_xyz, const float *d_vtx_rgb, con
                              uint32_t *d_out_vtx_count, int32_t *d_out_tri, uint32_t *d_out_tri_count,
                              int32_t *d_error, void *stream);
 
+/* m4 -- smoothing of ONE triangle mesh (Open3D FilterSmoothSimple / FilterSmoothLaplacian / FilterSmoothTaubin; our
+ * restatement, oracle/d2pc_smooth_oracle.py).  The neighbours of a vertex are Open3D's adjacency sets (triangle
+ * (a, b, c) adds b, c to adj[a], a, c to adj[b], a, b to adj[c]), visited in ascending vertex id.  The float32 input
+ * is widened to float64, every pass reads the previous state (Jacobi) and the result is rounded to float32 once.
+ *   SIMPLE      p' = (p + sum_nb p_nb) / (1 + |adj|)
+ *   LAPLACIAN   w = 1 / (sqrt((dx dx + dy dy) + dz dz) + 1e-12) of p - p_nb, p' = p + lambda (sum w p_nb / sum w - p);
+ *               a vertex without neighbours stays as it is
+ *   TAUBIN      every iteration a LAPLACIAN pass with lambda_filter, then one with mu
+ * Every sum runs left to right from zero.  `scope` is a non-empty set of D2PC_SMOOTH_VERTEX / _NORMAL / _COLOR
+ * (Open3D's FilterScope); colours and normals take the positions' weights; normals are filtered only when given and
+ * are not renormalised; the other fields are copied.  0 iterations copy everything.
+ *   d_vtx_xyz/rgb     float32 [vertices, 3]; d_vtx_normals float64 [vertices, 3] or NULL; d_tri int32 [triangles, 3]
+ *   d_scratch         d2pc_mesh_smooth_scratch_bytes(vertices, triangles) bytes, 256-byte aligned
+ *   d_out_xyz/rgb     float32 [vertices, 3]; d_out_normals float64 [vertices, 3] (NULL exactly when d_vtx_normals
+ *                     is); outputs must not overlap the inputs
+ *   d_error           int32 [1]: bit 1 = a triangle id outside [0, vertices), bit 2 = a non-finite coordinate (or
+ *                     colour / normal in the scope), bit 4 = a loop bound was exhausted (an internal failure, never
+ *                     expected); any error leaves the filtered outputs undefined
+ * triangles <= 2^25 and vertices <= 2^31, else D2PC_ERR_UNSUPPORTED.  lambda_filter and mu finite; an unknown method
+ * or scope and every other argument error are returned before any launch.  No floating-point atomics: the result
+ * repeats bit for bit.  The call does not synchronise. */
+enum { D2PC_SMOOTH_SIMPLE = 0, D2PC_SMOOTH_LAPLACIAN = 1, D2PC_SMOOTH_TAUBIN = 2 };
+enum { D2PC_SMOOTH_VERTEX = 1, D2PC_SMOOTH_NORMAL = 2, D2PC_SMOOTH_COLOR = 4 };
+int d2pc_mesh_smooth_scratch_bytes(uint32_t vertices, uint32_t triangles, size_t *bytes);
+int d2pc_mesh_smooth_enqueue(const float *d_vtx_xyz, const float *d_vtx_rgb, const double *d_vtx_normals,
+                             uint32_t vertices, const int32_t *d_tri, uint32_t triangles, int method,
+                             uint32_t iterations, double lambda_filter, double mu, uint32_t scope,
+                             void *d_scratch, size_t scratch_bytes, float *d_out_xyz, float *d_out_rgb,
+                             double *d_out_normals, int32_t *d_error, void *stream);
+
+/* m4 -- vertex normals of ANY triangle mesh, m1's rule (Open3D ComputeVertexNormals): the unnormalised
+ * (p1 - p0) x (p2 - p0) of every triangle in float64, summed per vertex in ascending triangle order once per corner,
+ * then v / sqrt(v.v), (0, 0, 1) for a zero sum.  Equals d2pc_grid_mesh_enqueue's normals bit for bit.
+ *   d_vtx_xyz float32 [vertices, 3]; d_tri int32 [triangles, 3]; d_out_normals float64 [vertices, 3]
+ *   d_scratch d2pc_mesh_vertex_normals_scratch_bytes(vertices, triangles) bytes, 256-byte aligned
+ *   d_error   as d2pc_mesh_smooth_enqueue's (bit 2: a non-finite coordinate)
+ * The size limits are those of d2pc_mesh_smooth_enqueue.  Argument errors are returned before any launch; the call
+ * does not synchronise. */
+int d2pc_mesh_vertex_normals_scratch_bytes(uint32_t vertices, uint32_t triangles, size_t *bytes);
+int d2pc_mesh_vertex_normals_enqueue(const float *d_vtx_xyz, uint32_t vertices, const int32_t *d_tri,
+                                     uint32_t triangles, void *d_scratch, size_t scratch_bytes,
+                                     double *d_out_normals, int32_t *d_error, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
