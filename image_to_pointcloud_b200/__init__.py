@@ -10,6 +10,7 @@ The package holds only what that path needs: ``csrc/`` (CUDA kernels + the C ABI
 from .api import create_depth_preview, depth_preview_bgr, depth_to_point_cloud, depth_to_point_cloud_batch
 from .engine import DENSITY_STEP, BatchStream, EmitResult, FrameEngine, reference_intrinsics, shard_frames
 from .hostpipe import HostFramePipeline, MultiGpuPipeline
+from .cluster import cluster_dbscan, remove_radius_outlier, remove_small_clusters
 from ._lib import D2pcConfig, D2pcError, D2pcFrameParams, load_library
 from .mesh import (TriangleMesh, cluster_connected_triangles, compute_vertex_normals, depth_to_mesh,
                    filter_smooth_laplacian, filter_smooth_simple, filter_smooth_taubin, grid_mesh,
@@ -29,6 +30,6 @@ __all__ = [
     "estimate_normals", "grid_mesh", "depth_to_mesh", "TriangleMesh", "ply_face_records", "mesh_ply_bytes",
     "save_mesh_ply", "simplify_mesh", "cluster_connected_triangles", "remove_triangles_by_mask",
     "remove_small_components", "filter_smooth_simple", "filter_smooth_laplacian", "filter_smooth_taubin",
-    "compute_vertex_normals",
+    "compute_vertex_normals", "cluster_dbscan", "remove_radius_outlier", "remove_small_clusters",
 ]
 __version__ = "0.1.0"

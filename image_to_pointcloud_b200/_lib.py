@@ -16,6 +16,7 @@ MESH_REMOVE_UNREFERENCED, MESH_NORMALS = 1, 2
 SIMPLIFY_QUADRIC, SIMPLIFY_NORMALS = 1, 2
 SMOOTH_SIMPLE, SMOOTH_LAPLACIAN, SMOOTH_TAUBIN = 0, 1, 2
 SMOOTH_VERTEX, SMOOTH_NORMAL, SMOOTH_COLOR = 1, 2, 4
+CLUSTER_ERR_NONFINITE, CLUSTER_ERR_GRID, CLUSTER_ERR_BOUND = 1, 2, 4
 
 EXPORTS = [
     "d2pc_abi_version", "d2pc_error_string", "d2pc_last_cuda_error", "d2pc_workspace_bytes",
@@ -30,6 +31,7 @@ EXPORTS = [
     "d2pc_mesh_components_scratch_bytes", "d2pc_mesh_components_enqueue", "d2pc_mesh_filter_scratch_bytes",
     "d2pc_mesh_filter_enqueue", "d2pc_mesh_smooth_scratch_bytes", "d2pc_mesh_smooth_enqueue",
     "d2pc_mesh_vertex_normals_scratch_bytes", "d2pc_mesh_vertex_normals_enqueue",
+    "d2pc_cluster_scratch_bytes", "d2pc_radius_outlier_enqueue", "d2pc_dbscan_enqueue",
     "d2pc_path_create", "d2pc_path_destroy", "d2pc_path_enqueue", "d2pc_path_trace_offset",
 ]
 
@@ -134,6 +136,11 @@ def load_library(path: str | None = None) -> C.CDLL:
                                              C.c_double, C.c_uint32, vp, C.c_size_t, vp, vp, vp, vp, vp]
     lib.d2pc_mesh_vertex_normals_scratch_bytes.argtypes = [C.c_uint32, C.c_uint32, C.POINTER(C.c_size_t)]
     lib.d2pc_mesh_vertex_normals_enqueue.argtypes = [vp, C.c_uint32, vp, C.c_uint32, vp, C.c_size_t, vp, vp, vp]
+    lib.d2pc_cluster_scratch_bytes.argtypes = [C.c_uint32, C.POINTER(C.c_size_t)]
+    lib.d2pc_radius_outlier_enqueue.argtypes = [vp, vp, vp, C.c_uint32, vp, C.c_int32, C.c_double, vp, C.c_size_t, vp,
+                                                vp, vp, vp, vp]
+    lib.d2pc_dbscan_enqueue.argtypes = [vp, vp, vp, C.c_uint32, vp, C.c_double, C.c_int32, C.c_uint32, vp, C.c_size_t,
+                                        vp, vp, vp, vp, vp, vp, vp]
     lib.d2pc_path_trace_offset.argtypes = [cfgp, C.POINTER(C.c_size_t)]
     lib.d2pc_path_create.argtypes = [C.POINTER(vp)]
     lib.d2pc_path_destroy.argtypes = [vp]

@@ -16,7 +16,7 @@ BUILD_DIR = os.path.join(PKG_DIR, "_build")
 LIB_PATH = os.path.join(BUILD_DIR, "libd2pc.so")
 SOURCES = ["d2pc_api.cu", "d2pc_stats.cu", "d2pc_emit.cu", "d2pc_path.cu", "d2pc_voxel.cu", "d2pc_serialise.cu", "d2pc_sor.cu",
            "d2pc_normals.cu", "d2pc_mesh.cu", "d2pc_simplify.cu", "d2pc_components.cu",
-           "d2pc_smooth.cu"]
+           "d2pc_smooth.cu", "d2pc_cluster.cu"]
 HEADERS = ["d2pc_math.h", "d2pc_format.h", "d2pc_device.cuh", "d2pc_stats_dev.cuh", "d2pc_emit_dev.cuh", "d2pc_grid.cuh",
            "d2pc_scan.cuh", "d2pc_components.h", "d2pc_smooth.h",
            os.path.join("..", "..", "include", "d2pc.h")]

@@ -100,6 +100,17 @@ inline SorWs sor_ws(void *base, uint32_t n_rows) {
 int sor_grid_build(const SorWs &w, const float *d_xyz, const uint32_t *d_count, const float *d_bounds,
                    uint32_t capacity_rows, cudaStream_t st);
 
+// The same grid with the cell size `cs` given (begin, clear, count, scan, scatter; no heavy cells).  *d_err gets
+// D2PC_CLUSTER_ERR_GRID when an axis of the box would need kSorCellLimit cells or more, else 0.
+constexpr double kSorCellLimit = 1048574.0;   // cells per axis below which sor_cell_coords never clamps
+int sor_grid_build_fixed(const SorWs &w, const float *d_xyz, const uint32_t *d_count, const float *d_bounds, double cs,
+                         uint32_t capacity_rows, uint32_t *d_err, cudaStream_t st);
+
+// Ordered compaction of the rows with 0 < avg[i] < hdr->thr (keep counts per tile, scan, copy) into d_out_* with
+// their source rows; *d_out_count = kept rows.
+int sor_compact(const SorWs &w, const float *d_xyz, const float *d_rgb, float *d_out_xyz, float *d_out_rgb,
+                uint32_t *d_out_index, uint32_t *d_out_count, uint32_t capacity_rows, cudaStream_t st);
+
 #if defined(__CUDACC__)
 __device__ __forceinline__ uint32_t sor_hash(unsigned long long k) {
   k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;

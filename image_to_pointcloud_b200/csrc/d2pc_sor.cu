@@ -56,6 +56,33 @@ __global__ void sor_begin_kernel(SorWs w, const uint32_t *count, const float *bo
   h->heavy_total = 0;
 }
 
+// Grid of one cell size given by the caller (density clustering, d2pc_cluster.cu).  Sets *err to
+// D2PC_CLUSTER_ERR_GRID when an axis would need kSorCellLimit cells or more: sor_cell_coords clamps beyond that,
+// and a clamped cell would merge points that are far apart.
+__global__ void sor_fixed_begin_kernel(SorWs w, const uint32_t *count, const float *bounds, double cs, uint32_t *err) {
+  if (threadIdx.x != 0) return;
+  SorHeader *h = w.hdr;
+  const uint32_t n = *count;
+  h->n = n;
+  double mx = 0.0;
+  bool fits = true;
+  for (int a = 0; a < 3; ++a) {
+    const double lo = (double)bounds[a], hi = (double)bounds[3 + a];
+    h->mn[a] = (n > 0 && lo == lo) ? lo : 0.0;
+    h->ext[a] = (n > 0 && hi == hi && lo == lo && hi > lo) ? hi - lo : 0.0;
+    if (h->ext[a] > mx) mx = h->ext[a];
+    const double q = h->ext[a] / cs;
+    fits = fits && q < kSorCellLimit;
+    h->dim[a] = q < kSorCellLimit ? (int32_t)floor(q) + 1 : (int32_t)kSorCellLimit;
+  }
+  h->h = cs;
+  h->chosen = 0;
+  h->slack = 1e-9 * mx + 1e-300;
+  h->n_heavy = 0;
+  h->heavy_total = 0;
+  *err = fits ? 0u : (uint32_t)D2PC_CLUSTER_ERR_GRID;
+}
+
 __global__ void sor_clear_kernel(SorWs w) {
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < w.cap; i += (size_t)gridDim.x * blockDim.x) {
     w.keys[i] = kSorEmpty;
@@ -597,6 +624,40 @@ int sor_grid_build(const SorWs &w, const float *d_xyz, const uint32_t *d_count, 
   return D2PC_OK;
 }
 
+int sor_grid_build_fixed(const SorWs &w, const float *d_xyz, const uint32_t *d_count, const float *d_bounds, double cs,
+                         uint32_t capacity_rows, uint32_t *d_err, cudaStream_t st) {
+  const uint32_t row_blocks = (capacity_rows + kSorThreads - 1) / kSorThreads;
+  const uint32_t stride_blocks = min(row_blocks, 148u * 16u);
+  const uint32_t cell_blocks = w.cap / kSorScanThreads + 1;
+  sor_fixed_begin_kernel<<<1, 32, 0, st>>>(w, d_count, d_bounds, cs, d_err);
+  D2PC_CHECK_LAUNCH();
+  sor_clear_kernel<<<148 * 8, 256, 0, st>>>(w);
+  D2PC_CHECK_LAUNCH();
+  sor_count_kernel<<<stride_blocks, kSorThreads, 0, st>>>(w, d_xyz);
+  D2PC_CHECK_LAUNCH();
+  sor_scan1_kernel<<<cell_blocks, kSorScanThreads, 0, st>>>(w);
+  D2PC_CHECK_LAUNCH();
+  sor_scan2_kernel<<<1, kSorScanThreads, 0, st>>>(w);
+  D2PC_CHECK_LAUNCH();
+  sor_scan3_kernel<<<cell_blocks, kSorScanThreads, 0, st>>>(w);
+  D2PC_CHECK_LAUNCH();
+  sor_scatter_kernel<<<stride_blocks, kSorThreads, 0, st>>>(w, d_xyz);
+  D2PC_CHECK_LAUNCH();
+  return D2PC_OK;
+}
+
+int sor_compact(const SorWs &w, const float *d_xyz, const float *d_rgb, float *d_out_xyz, float *d_out_rgb,
+                uint32_t *d_out_index, uint32_t *d_out_count, uint32_t capacity_rows, cudaStream_t st) {
+  const uint32_t row_blocks = (capacity_rows + kSorThreads - 1) / kSorThreads;
+  sor_keep_count_kernel<<<row_blocks, kSorThreads, 0, st>>>(w);
+  D2PC_CHECK_LAUNCH();
+  sor_tile_scan_kernel<<<1, kSorScanThreads, 0, st>>>(w, d_out_count);
+  D2PC_CHECK_LAUNCH();
+  sor_compact_kernel<<<row_blocks, kSorThreads, 0, st>>>(w, d_xyz, d_rgb, d_out_xyz, d_out_rgb, d_out_index);
+  D2PC_CHECK_LAUNCH();
+  return D2PC_OK;
+}
+
 }  // namespace d2pc
 
 using namespace d2pc;
@@ -635,11 +696,5 @@ extern "C" int d2pc_sor_enqueue(const float *d_xyz, const float *d_rgb, const ui
     sor_finish_kernel<<<1, 32, 0, st>>>(w, pass, partial, std_ratio, d_stats);
     D2PC_CHECK_LAUNCH();
   }
-  sor_keep_count_kernel<<<row_blocks, kSorThreads, 0, st>>>(w);
-  D2PC_CHECK_LAUNCH();
-  sor_tile_scan_kernel<<<1, kSorScanThreads, 0, st>>>(w, d_out_count);
-  D2PC_CHECK_LAUNCH();
-  sor_compact_kernel<<<row_blocks, kSorThreads, 0, st>>>(w, d_xyz, d_rgb, d_out_xyz, d_out_rgb, d_out_index);
-  D2PC_CHECK_LAUNCH();
-  return D2PC_OK;
+  return sor_compact(w, d_xyz, d_rgb, d_out_xyz, d_out_rgb, d_out_index, d_out_count, capacity_rows, st);
 }

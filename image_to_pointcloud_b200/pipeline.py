@@ -1,7 +1,8 @@
 """Everything process_image_pipeline does between the depth network and the job result
 (reference backend/app.py:468-559) in ONE device-resident pass:
 
-    depth_to_point_cloud (:468-476) -> refine_point_cloud (:479) -> preview decimation (:495-506)
+    depth_to_point_cloud (:468-476) -> refine_point_cloud (:479)
+    [-> remove_small_clusters of the refined rows (row f5), with cluster_eps] -> preview decimation (:495-506)
     -> save_point_cloud (:537) -> generate_gis_metadata bounds (:393-400)
     [-> estimate_normals, the mesh builder's first step (:271-308), with normals=True]
     [-> grid_mesh of the refined lattice rows, the mesh PLY (row m1), with mesh=True]
@@ -24,7 +25,7 @@ from typing import Optional
 import numpy as np
 import torch
 
-from . import _lib, writers
+from . import _lib, cluster, writers
 from ._lib import check
 from .api import _engine_for, _image_channels, _to_host, bounds_dict, check_depth_dtype
 from .engine import DENSITY_STEP
@@ -41,7 +42,8 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
                       max_preview: int = writers.MAX_PREVIEW, return_arrays: bool = True, normals: bool = False,
                       normals_knn: int = 30, mesh: bool = False, mesh_max_angle: float = 85.0, mesh_max_edge=None,
                       mesh_preview_voxel: Optional[float] = None, mesh_min_triangles: Optional[int] = None,
-                      mesh_smooth_iterations: Optional[int] = None, device=None) -> dict:
+                      mesh_smooth_iterations: Optional[int] = None, cluster_eps: Optional[float] = None,
+                      cluster_min_points: int = 10, cluster_min_size: int = 1, device=None) -> dict:
     """Returns a dict with ``points`` / ``colors`` (host float32 [M,3], if ``return_arrays``), ``point_count``,
     ``preview_points`` / ``preview_colors`` (nested lists as app.py:505-506), ``bounds`` (app.py:393-400),
     and either ``filepath`` (``filename`` given: the file the reference's writer would have put into
@@ -59,7 +61,11 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
     smoothed) mesh is also simplified for a preview (``simplify_mesh(mesh, mesh_preview_voxel)``, average
     contraction): ``mesh_preview_vertex_count``,
     ``mesh_preview_triangle_count`` and either ``mesh_preview_filepath`` (outputs/<filename>_mesh_preview.ply) or
-    ``mesh_preview_file_bytes``."""
+    ``mesh_preview_file_bytes``.  With ``cluster_eps`` the (refined) rows are clustered (``remove_small_clusters(
+    points, colors, eps=cluster_eps, min_points=cluster_min_points, min_size=cluster_min_size)``) before the normals,
+    the preview, the file, the bounds and the mesh: noise and clusters below ``cluster_min_size`` points are dropped
+    from all of them (the mesh's lattice keep mask composes both removals).  It adds ``cluster_count`` (before the
+    removal) and ``cluster_removed_point_count``."""
     DENSITY_STEP[density]  # KeyError first, like the reference
     if mesh:   # mesh argument errors before any device work
         _cos2(mesh_max_angle), _max_edge(mesh_max_edge)
@@ -75,6 +81,10 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
         if not mesh:
             raise ValueError("mesh_smooth_iterations needs mesh=True")
         check_iterations(mesh_smooth_iterations)
+    if cluster_eps is not None:
+        cluster_eps = cluster.check_eps(cluster_eps, "cluster_eps")
+        cluster_min_points = cluster.check_min_points(cluster_min_points, "cluster_min_points")
+        cluster_min_size = cluster.check_min_size(cluster_min_size, "cluster_min_size")
     lib = _lib.load_library()
     img_h, img_w = image.shape[:2]
     dep_h, dep_w = depth.shape[:2]
@@ -93,8 +103,14 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
         lat_xyz, lat_rgb, kept = xyz, rgb, None   # the emit rows are the unmasked lattice
         if refine and n > 0:
             xyz, rgb, kept, _ = statistical_outlier_removal(xyz, rgb, nb_neighbors, std_ratio, return_device=True)
+        out = {}
+        if cluster_eps is not None:
+            r = cluster._run(xyz, rgb, cluster_eps, min_points=cluster_min_points, min_size=cluster_min_size)
+            out["cluster_count"], out["cluster_removed_point_count"] = r["clusters"], int(xyz.shape[0]) - r["kept"]
+            xyz, rgb = r["xyz"], r["rgb"]
+            kept = r["index"] if kept is None else kept[r["index"].to(torch.int64)]
         m = int(xyz.shape[0])
-        out = {"point_count": m}
+        out["point_count"] = m
         nrm = estimate_normals(xyz, knn=normals_knn, return_device=True) if normals else None
         if return_arrays:
             out["points"], out["colors"] = _to_host(xyz), _to_host(rgb)   # pinned D2H at PCIe speed

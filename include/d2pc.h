@@ -31,6 +31,8 @@
  *   a11 emission (:246), ax-1 depth-range mask + compaction   -> d2pc_emit_enqueue
  *   ax-2 voxel-grid down-sampling (north-star extension)      -> d2pc_voxel_enqueue
  *   f1 refine_point_cloud (:252-269, Open3D SOR)               -> d2pc_sor_enqueue
+ *   f5 density clustering (Open3D cluster_dbscan,
+ *      remove_radius_outlier)                                  -> d2pc_dbscan_enqueue, d2pc_radius_outlier_enqueue
  *   f3 preview stride (:495-506), save_xyz/las/ply (:329-389) -> d2pc_preview_rows_enqueue,
  *                                                               d2pc_xyz_text_*, d2pc_las_records_enqueue,
  *                                                               d2pc_ply_records_enqueue
@@ -298,6 +300,40 @@ int d2pc_sor_enqueue(const float *d_xyz, const float *d_rgb, const uint32_t *d_c
                      const float *d_bounds, int32_t nb_neighbors, double std_ratio, void *d_scratch,
                      size_t scratch_bytes, float *d_out_xyz, float *d_out_rgb, uint32_t *d_out_index,
                      uint32_t *d_out_count, double *d_stats, void *stream);
+
+/* f5 -- density clustering of ONE cloud (Open3D ClusterDBSCAN and RemoveRadiusOutliers; spec in
+ * oracle/d2pc_cluster_oracle.py).  Point j is a neighbour of point i when d2(i, j) < eps * eps (strict), d2 summed
+ * axis by axis in float64 from the float32 rows; the point itself is a neighbour.  A uniform grid of cell side
+ * eps / 2 * (1 + 2^-20) holds the rows, so every neighbour lies in the 5 x 5 x 5 cells around a row's own cell.
+ *   d_bounds       float32 [6] min/max of the rows (d2pc_rows_bounds_enqueue)
+ *   d_scratch      d2pc_cluster_scratch_bytes(capacity_rows) bytes, 256-byte aligned
+ *   d_out_xyz/rgb  float32 [capacity_rows, 3] kept rows in input order (d_rgb / d_out_rgb may both be NULL);
+ *                  d_out_index uint32 [capacity_rows] their source rows, or NULL
+ *   d_out_counts   uint32 [4] = kept rows, error bits (D2PC_CLUSTER_ERR_*), clusters (DBSCAN only), 0
+ * The error bits are set on the device: a row with a non-finite coordinate; an eps so small that an axis of the
+ * bounding box needs 1048574 cells or more (the grid cannot hold the cloud: the call refuses it rather than return
+ * a wrong result); an exhausted loop bound (an internal failure, never expected).  Any error leaves the other
+ * outputs undefined.  No floating-point atomics: the result repeats bit for bit.  Argument errors are returned
+ * before any launch; the call does not synchronise. */
+enum { D2PC_CLUSTER_ERR_NONFINITE = 1, D2PC_CLUSTER_ERR_GRID = 2, D2PC_CLUSTER_ERR_BOUND = 4 };
+int d2pc_cluster_scratch_bytes(uint32_t capacity_rows, size_t *bytes);
+/* Row i is kept iff it has more than nb_points neighbours within radius (itself counted).  nb_points >= 1, radius
+ * finite and > 0 with radius * radius > 0. */
+int d2pc_radius_outlier_enqueue(const float *d_xyz, const float *d_rgb, const uint32_t *d_count,
+                                uint32_t capacity_rows, const float *d_bounds, int32_t nb_points, double radius,
+                                void *d_scratch, size_t scratch_bytes, float *d_out_xyz, float *d_out_rgb,
+                                uint32_t *d_out_index, uint32_t *d_out_counts, void *stream);
+/* DBSCAN: a row is core when it has at least min_points neighbours; clusters are the connected components of the
+ * cores under the neighbour relation, numbered 0, 1, ... by their lowest core row; a non-core row takes the lowest
+ * cluster among its core neighbours, else -1.
+ *   d_out_labels   int32 [capacity_rows]; d_out_sizes uint32 [capacity_rows], the rows of every cluster
+ *   min_size       with d_out_xyz set, the rows of clusters of at least min_size rows are kept (noise is dropped);
+ *                  d_out_xyz NULL: no compaction (d_out_rgb and d_out_index NULL too)
+ * eps finite and > 0 with eps * eps > 0; min_points >= 0; min_size >= 1. */
+int d2pc_dbscan_enqueue(const float *d_xyz, const float *d_rgb, const uint32_t *d_count, uint32_t capacity_rows,
+                        const float *d_bounds, double eps, int32_t min_points, uint32_t min_size, void *d_scratch,
+                        size_t scratch_bytes, int32_t *d_out_labels, uint32_t *d_out_sizes, float *d_out_xyz,
+                        float *d_out_rgb, uint32_t *d_out_index, uint32_t *d_out_counts, void *stream);
 
 /* Point normals (Open3D PointCloud::EstimateNormals with fast_normal_computation, then
  * OrientNormalsTowardsCameraLocation) on ONE frame's rows, through the same grid as statistical outlier removal:
