@@ -20,6 +20,7 @@ from typing import Dict, Optional, Sequence, Tuple
 import numpy as np
 import torch
 
+from . import _device
 from .engine import DENSITY_STEP, MAX_SMOOTH_KSIZE, EmitResult, FrameEngine, smoothing_kernel
 
 logger = logging.getLogger(__name__)
@@ -179,15 +180,36 @@ def _run_locked(eng, st, image, depth, img_c, dep_h, dep_w, density, invert, dep
             vxyz, vrgb, vidx, vcount = eng.voxel_downsample(cfg, res, float(voxel_size),
                                                             want_index=return_voxel_index, stream=stream)
             n = int(vcount.cpu()[0])
-            out = (_unpin(_to_host(vxyz[0, :n]), pinned), _unpin(_to_host(vrgb[0, :n]), pinned))
+            out = (_unpin(_device.pinned(vxyz[0, :n]), pinned), _unpin(_device.pinned(vrgb[0, :n]), pinned))
             if return_voxel_index:
                 out = out + (vidx[0, :n].cpu().numpy(),)
             return out
         n = int(res.count.cpu()[0])
-        out = (_unpin(_to_host(res.xyz[0, :n]), pinned), _unpin(_to_host(res.rgb[0, :n]), pinned))
+        out = (_unpin(_device.pinned(res.xyz[0, :n]), pinned), _unpin(_device.pinned(res.rgb[0, :n]), pinned))
         if return_bounds:
             out = out + (bounds_dict(res.bounds[0].cpu().numpy()),)
         return out
+
+
+def _lattice_emit(image: np.ndarray, depth: np.ndarray, density: str, invert: bool, depth_scale: float, smooth: bool,
+                  smooth_ksize: int, fov: Optional[float], device):
+    """The unmasked emit of ``depth_to_point_cloud`` (same positional arguments) left on the device, for the stages
+    that continue from it: -> (device, xyz, rgb, n), the ``n`` lattice rows in this call's own tensors.  The engine's
+    lock is held while the engine runs; what the caller does with the rows does not need it."""
+    img_h, img_w = image.shape[:2]
+    dep_h, dep_w = depth.shape[:2]
+    check_depth_dtype(depth, int(img_h), int(img_w))
+    img_c = _image_channels(image)
+    eng = _engine_for(int(img_h), int(img_w), img_c, int(dep_h), int(dep_w), device)
+    dev = eng.device
+    cfg = eng.make_config(density=density, invert=invert, depth_scale=float(depth_scale), fov=fov)
+    n = eng.points_per_frame(cfg)   # the emit is unmasked: every lattice point is a row
+    with eng._staging["lock"], torch.cuda.device(dev):
+        d = torch.from_numpy(np.ascontiguousarray(depth, dtype=np.float32).reshape(1, dep_h, dep_w)).to(dev)
+        im = torch.from_numpy(np.ascontiguousarray(image).reshape(1, img_h, img_w, -1)).to(dev) if img_c >= 3 else None
+        res = eng.process(cfg, d, im, stream=torch.cuda.current_stream(dev),
+                          smooth_ksize=(smooth_ksize if smooth else None))
+    return dev, res.xyz[0, :n], res.rgb[0, :n], n
 
 
 DEPTH_PREVIEW_MAX = 2048  # reference backend/app.py:44
@@ -233,14 +255,6 @@ def bounds_dict(b6: np.ndarray) -> dict:
     also the LAS offsets of save_las, app.py:352), from the min/max reduction fused into emit."""
     return {"minX": float(b6[0]), "maxX": float(b6[3]), "minY": float(b6[1]), "maxY": float(b6[4]),
             "minZ": float(b6[2]), "maxZ": float(b6[5])}
-
-
-def _to_host(t: torch.Tensor) -> np.ndarray:
-    """Device rows -> a fresh C-contiguous float32 NumPy array (pinned host memory from torch's
-    caching host allocator, so the copy runs at PCIe speed; the array owns its buffer)."""
-    host = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
-    host.copy_(t, non_blocking=False)
-    return host.numpy()
 
 
 def depth_to_point_cloud_batch(images: Sequence[np.ndarray], depths: Sequence[np.ndarray],

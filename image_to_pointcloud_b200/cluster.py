@@ -9,15 +9,14 @@ count) per call.
 """
 from __future__ import annotations
 
-import ctypes as C
 import math
 
 import numpy as np
 import torch
 
 from . import _lib
+from ._device import device_rows, ptr, raise_errors, row_bounds, scratch, stream, to_host
 from ._lib import check
-from .writers import _device_rows, _stream
 
 GRID_CELL_LIMIT = 1048574.0    # cells per axis the device grid holds (d2pc_grid.cuh, kSorCellLimit)
 RADIUS_MESSAGE = "Illegal input parameters, number of points and radius must be positive"
@@ -67,12 +66,10 @@ def _check_host_points(points, eps: float) -> None:
 
 
 def _raise_for(err: int, eps: float) -> None:
-    if err & _lib.CLUSTER_ERR_NONFINITE:
-        raise ValueError("points must be finite")
-    if err & _lib.CLUSTER_ERR_GRID:
-        raise ValueError(_grid_message(eps))
-    if err:
-        raise RuntimeError(f"density clustering failed on the device (error bits {err})")
+    if err & _lib.CLUSTER_ERR_NONFINITE:   # a non-finite row also spoils the bounds the grid is sized from
+        err &= ~_lib.CLUSTER_ERR_GRID
+    raise_errors(err, ((_lib.CLUSTER_ERR_NONFINITE, "points must be finite"),
+                       (_lib.CLUSTER_ERR_GRID, _grid_message(eps))), "density clustering")
 
 
 def _run(points, colors, eps, *, min_points=None, min_size=None, nb_points=None, compact=True, device=None):
@@ -80,7 +77,7 @@ def _run(points, colors, eps, *, min_points=None, min_size=None, nb_points=None,
     labels / sizes (DBSCAN), xyz / rgb / index (compact), and the host ints kept, clusters."""
     lib = _lib.load_library()
     has_colors = colors is not None and len(colors) == len(points)
-    xyz, rgb, count, n = _device_rows(points, colors if has_colors else None, device)
+    xyz, rgb, count, n = device_rows(points, colors if has_colors else None, device)
     dev = xyz.device
     out = {"kept": 0, "clusters": 0}
     with torch.cuda.device(dev):
@@ -90,30 +87,24 @@ def _run(points, colors, eps, *, min_points=None, min_size=None, nb_points=None,
             out["xyz"], out["rgb"], out["index"] = xyz, (rgb if has_colors else None), torch.zeros(0, dtype=torch.int32,
                                                                                                  device=dev)
             return out
-        nb = C.c_size_t(0)
-        check(lib.d2pc_cluster_scratch_bytes(n, C.byref(nb)), "d2pc_cluster_scratch_bytes")
-        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
-        keys = torch.empty(6, dtype=torch.int32, device=dev)
-        bounds = torch.empty(6, dtype=torch.float32, device=dev)
-        s = _stream(dev)
-        check(lib.d2pc_rows_bounds_enqueue(xyz.data_ptr(), count.data_ptr(), n, keys.data_ptr(), bounds.data_ptr(), s),
-              "d2pc_rows_bounds_enqueue")
+        buf = scratch(lib.d2pc_cluster_scratch_bytes, n, dev=dev)
+        bounds = row_bounds(xyz, count, n, dev)
+        s = stream(dev)
         counts = torch.zeros(4, dtype=torch.int32, device=dev)
         oxyz = torch.empty_like(xyz) if compact else None
         orgb = torch.empty_like(rgb) if compact and has_colors else None
         oidx = torch.empty(n, dtype=torch.int32, device=dev) if compact else None
-        ptr = (lambda t: t.data_ptr() if t is not None else None)
         if nb_points is None:
             labels = torch.empty(n, dtype=torch.int32, device=dev)
             sizes = torch.empty(n, dtype=torch.int32, device=dev)
             check(lib.d2pc_dbscan_enqueue(xyz.data_ptr(), rgb.data_ptr() if orgb is not None else None, count.data_ptr(),
                                           n, bounds.data_ptr(), eps, min_points, min_size if min_size else 1,
-                                          scratch.data_ptr(), scratch.numel(), labels.data_ptr(), sizes.data_ptr(),
+                                          buf.data_ptr(), buf.numel(), labels.data_ptr(), sizes.data_ptr(),
                                           ptr(oxyz), ptr(orgb), ptr(oidx), counts.data_ptr(), s), "d2pc_dbscan_enqueue")
         else:
             check(lib.d2pc_radius_outlier_enqueue(xyz.data_ptr(), rgb.data_ptr() if has_colors else None,
                                                   count.data_ptr(), n, bounds.data_ptr(), nb_points, eps,
-                                                  scratch.data_ptr(), scratch.numel(), ptr(oxyz), ptr(orgb), ptr(oidx),
+                                                  buf.data_ptr(), buf.numel(), ptr(oxyz), ptr(orgb), ptr(oidx),
                                                   counts.data_ptr(), s), "d2pc_radius_outlier_enqueue")
         kept, err, clusters, _ = (int(v) for v in counts.cpu())
         _raise_for(err, eps)
@@ -126,10 +117,8 @@ def _run(points, colors, eps, *, min_points=None, min_size=None, nb_points=None,
 
 
 def _rows(r, return_device: bool):
-    if return_device:
-        return r["xyz"], r["rgb"], r["index"]
-    return (r["xyz"].cpu().numpy(), r["rgb"].cpu().numpy() if r["rgb"] is not None else None,
-            r["index"].cpu().numpy().astype(np.int64))
+    xyz, rgb, index = to_host((r["xyz"], r["rgb"], r["index"]), return_device)
+    return xyz, rgb, (index if return_device else index.astype(np.int64))
 
 
 def cluster_dbscan(points, eps: float, min_points: int, *, device=None, return_device: bool = False):
@@ -138,7 +127,7 @@ def cluster_dbscan(points, eps: float, min_points: int, *, device=None, return_d
     eps, min_points = check_eps(eps), check_min_points(min_points)
     _check_host_points(points, eps)
     r = _run(points, None, eps, min_points=min_points, compact=False, device=device)
-    return r["labels"] if return_device else r["labels"].cpu().numpy()
+    return to_host(r["labels"], return_device)
 
 
 def remove_radius_outlier(points, colors=None, *, nb_points: int, radius: float, device=None,

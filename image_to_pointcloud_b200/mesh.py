@@ -29,7 +29,6 @@ any mesh, e.g. to take the terraces of a monocular depth map out of the lattice 
 """
 from __future__ import annotations
 
-import ctypes as C
 import math
 from typing import NamedTuple, Optional
 
@@ -37,11 +36,11 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._device import device_for, device_rows, ptr, raise_errors, scratch, stream, to_host, upload
 from ._lib import check
-from .api import _engine_for, _image_channels, check_depth_dtype
+from .api import _lattice_emit
 from .engine import DENSITY_STEP
 from .refine import statistical_outlier_removal
-from .writers import _device_rows, _stream
 
 
 class TriangleMesh(NamedTuple):
@@ -83,7 +82,7 @@ def grid_mesh(points, colors, lattice_shape, *, keep=None, max_edge=None, max_an
         raise ValueError("lattice_shape must be (R, C) with R, C >= 1 and R * C < 2^31")
     cos2, me = _cos2(max_angle), _max_edge(max_edge)
     lib = _lib.load_library()
-    xyz, rgb, _, n = _device_rows(points, colors, device)
+    xyz, rgb, _, n = device_rows(points, colors, device)
     if n != R * Cc:
         raise ValueError(f"{n} rows do not form a {R} x {Cc} lattice")
     dev = xyz.device
@@ -95,9 +94,7 @@ def grid_mesh(points, colors, lattice_shape, *, keep=None, max_edge=None, max_an
             if keep_t.numel() != n:
                 raise ValueError("keep must have one entry per lattice row")
             keep_t = (keep_t != 0).to(torch.uint8).contiguous()
-        nb = C.c_size_t(0)
-        check(lib.d2pc_grid_mesh_scratch_bytes(R, Cc, C.byref(nb)), "d2pc_grid_mesh_scratch_bytes")
-        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+        buf = scratch(lib.d2pc_grid_mesh_scratch_bytes, R, Cc, dev=dev)
         vxyz = torch.empty((n, 3), dtype=torch.float32, device=dev)
         vrgb = torch.empty((n, 3), dtype=torch.float32, device=dev)
         vrow = torch.empty(n, dtype=torch.int32, device=dev)
@@ -106,17 +103,14 @@ def grid_mesh(points, colors, lattice_shape, *, keep=None, max_edge=None, max_an
         counts = torch.zeros(2, dtype=torch.int32, device=dev)   # vertices, triangles
         flags = (_lib.MESH_REMOVE_UNREFERENCED if remove_unreferenced else 0) | \
             (_lib.MESH_NORMALS if compute_normals else 0)
-        check(lib.d2pc_grid_mesh_enqueue(xyz.data_ptr(), rgb.data_ptr(), keep_t.data_ptr() if keep_t is not None else None,
-                                         R, Cc, me, cos2, flags, scratch.data_ptr(), scratch.numel(), vxyz.data_ptr(),
-                                         vrgb.data_ptr(), vrow.data_ptr(), vnrm.data_ptr() if vnrm is not None else None,
-                                         counts.data_ptr(), tri.data_ptr(), counts.data_ptr() + 4, _stream(dev)),
-              "d2pc_grid_mesh_enqueue")
+        check(lib.d2pc_grid_mesh_enqueue(xyz.data_ptr(), rgb.data_ptr(), ptr(keep_t), R, Cc, me, cos2, flags,
+                                         buf.data_ptr(), buf.numel(), vxyz.data_ptr(), vrgb.data_ptr(), vrow.data_ptr(),
+                                         ptr(vnrm), counts.data_ptr(), tri.data_ptr(), counts.data_ptr() + 4,
+                                         stream(dev)), "d2pc_grid_mesh_enqueue")
         nv, nt = (int(v) for v in counts.cpu())
         mesh = TriangleMesh(vxyz[:nv], vrgb[:nv], tri[:nt], vnrm[:nv] if vnrm is not None else None,
                             vrow[:nv].to(torch.int64))
-        if return_device:
-            return mesh
-        return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in mesh))
+        return to_host(mesh, return_device)
 
 
 CONTRACTIONS = ("average", "quadric")
@@ -131,15 +125,42 @@ def check_voxel_size(voxel_size) -> float:
     return vs
 
 
-def _device_array(x, dtype, cols, dev):
-    if isinstance(x, torch.Tensor):
-        t = x.to(dev)
-    else:
-        np_dtype = {torch.float32: np.float32, torch.float64: np.float64, torch.int32: np.int32, torch.int64: np.int64}
-        t = torch.from_numpy(np.ascontiguousarray(x, dtype=np_dtype[dtype])).to(dev)
-    if t.dtype != dtype:
-        raise ValueError(f"expected {dtype}, got {t.dtype}")
-    return (t.reshape(-1, cols) if cols else t.reshape(-1)).contiguous()
+def _mesh_inputs(mesh: TriangleMesh, dev, normals: bool = True):
+    """-> (xyz, rgb, triangles, vertex rows, normals or None) of ``mesh`` on ``dev``; with ``normals=False`` the mesh's
+    normals are left out."""
+    nv = len(mesh.vertices)
+    xyz = upload(mesh.vertices, torch.float32, 3, dev)
+    rgb = upload(mesh.colors, torch.float32, 3, dev)
+    tri = upload(mesh.triangles, torch.int32, 3, dev)
+    rows = upload(mesh.vertex_rows, torch.int64, 0, dev)
+    nrm = None if mesh.vertex_normals is None or not normals else upload(mesh.vertex_normals, torch.float64, 3, dev)
+    if len(rgb) != nv or len(rows) != nv or (nrm is not None and len(nrm) != nv):
+        raise ValueError("colors, vertex_rows and vertex_normals must have one row per vertex" if normals else
+                         "colors and vertex_rows must have one row per vertex")
+    return xyz, rgb, tri, rows, nrm
+
+
+def _reduce_mesh(scratch_bytes, enqueue, mesh: TriangleMesh, arg, flags: int, errors, where: str, dev,
+                 return_device: bool) -> TriangleMesh:
+    """One call of ``d2pc_mesh_simplify_enqueue`` or ``d2pc_mesh_filter_enqueue``: the same inputs, outputs (at most
+    the input's vertices and triangles) and word block (vertices, triangles, error) around an argument of their own,
+    ``arg`` (the voxel size, the keep mask)."""
+    nv, nt = len(mesh.vertices), len(mesh.triangles)
+    xyz, rgb, tri, rows, nrm = _mesh_inputs(mesh, dev)
+    buf = scratch(scratch_bytes, nv, nt, dev=dev)
+    oxyz = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+    orgb = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+    orow = torch.empty(nv, dtype=torch.int64, device=dev)
+    onrm = torch.empty((nv, 3), dtype=torch.float64, device=dev) if nrm is not None else None
+    otri = torch.empty((nt, 3), dtype=torch.int32, device=dev)
+    words = torch.zeros(3, dtype=torch.int32, device=dev)   # vertices, triangles, error
+    check(enqueue(ptr(xyz), ptr(rgb), ptr(nrm), ptr(rows), nv, ptr(tri), nt, arg, flags, buf.data_ptr(), buf.numel(),
+                  ptr(oxyz), ptr(orgb), ptr(onrm), ptr(orow), words.data_ptr(), ptr(otri), words.data_ptr() + 4,
+                  words.data_ptr() + 8, stream(dev)), enqueue.__name__)
+    kv, kt, err = (int(v) for v in words.cpu())
+    raise_errors(err, errors, where)
+    return to_host(TriangleMesh(oxyz[:kv], orgb[:kv], otri[:kt], onrm[:kv] if onrm is not None else None, orow[:kv]),
+                   return_device)
 
 
 def simplify_mesh(mesh: TriangleMesh, voxel_size: float, *, contraction: str = "average", device=None,
@@ -158,45 +179,12 @@ def simplify_mesh(mesh: TriangleMesh, voxel_size: float, *, contraction: str = "
     if nv >= 2 ** 24 or nt >= 2 ** 31:
         raise ValueError("simplify_mesh takes fewer than 2^24 vertices and 2^31 triangles")
     lib = _lib.load_library()
-    if not torch.cuda.is_available():
-        raise RuntimeError("image_to_pointcloud_b200 needs a CUDA device (no CPU fallback exists)")
-    if isinstance(mesh.vertices, torch.Tensor):
-        dev = mesh.vertices.device
-    else:
-        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+    dev = device_for(mesh.vertices, device)
+    flags = (_lib.SIMPLIFY_QUADRIC if contraction == "quadric" else 0) | \
+        (_lib.SIMPLIFY_NORMALS if mesh.vertex_normals is not None else 0)
     with torch.cuda.device(dev):
-        xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
-        rgb = _device_array(mesh.colors, torch.float32, 3, dev)
-        tri = _device_array(mesh.triangles, torch.int32, 3, dev)
-        rows = _device_array(mesh.vertex_rows, torch.int64, 0, dev)
-        nrm = None if mesh.vertex_normals is None else _device_array(mesh.vertex_normals, torch.float64, 3, dev)
-        if len(rgb) != nv or len(rows) != nv or (nrm is not None and len(nrm) != nv):
-            raise ValueError("colors, vertex_rows and vertex_normals must have one row per vertex")
-        nb = C.c_size_t(0)
-        check(lib.d2pc_mesh_simplify_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_simplify_scratch_bytes")
-        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
-        oxyz = torch.empty((nv, 3), dtype=torch.float32, device=dev)
-        orgb = torch.empty((nv, 3), dtype=torch.float32, device=dev)
-        orow = torch.empty(nv, dtype=torch.int64, device=dev)
-        onrm = torch.empty((nv, 3), dtype=torch.float64, device=dev) if nrm is not None else None
-        otri = torch.empty((nt, 3), dtype=torch.int32, device=dev)
-        words = torch.zeros(3, dtype=torch.int32, device=dev)   # vertices, triangles, error
-        flags = (_lib.SIMPLIFY_QUADRIC if contraction == "quadric" else 0) | (_lib.SIMPLIFY_NORMALS if nrm is not None else 0)
-
-        def ptr(t):
-            return t.data_ptr() if t is not None and t.numel() > 0 else None
-        check(lib.d2pc_mesh_simplify_enqueue(ptr(xyz), ptr(rgb), ptr(nrm), ptr(rows), nv, ptr(tri), nt, vs, flags,
-                                             scratch.data_ptr(), scratch.numel(), ptr(oxyz), ptr(orgb), ptr(onrm),
-                                             ptr(orow), words.data_ptr(), ptr(otri), words.data_ptr() + 4,
-                                             words.data_ptr() + 8, _stream(dev)),
-              "d2pc_mesh_simplify_enqueue")
-        kv, kt, err = (int(v) for v in words.cpu())
-        if err:
-            raise ValueError("; ".join(msg for bit, msg in _SIMPLIFY_ERRORS if err & bit))
-        out = TriangleMesh(oxyz[:kv], orgb[:kv], otri[:kt], onrm[:kv] if onrm is not None else None, orow[:kv])
-        if return_device:
-            return out
-        return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in out))
+        return _reduce_mesh(lib.d2pc_mesh_simplify_scratch_bytes, lib.d2pc_mesh_simplify_enqueue, mesh, vs, flags,
+                            _SIMPLIFY_ERRORS, "simplify_mesh", dev, return_device)
 
 
 _COMPONENT_ERRORS = ((1, "a triangle refers to a vertex that does not exist"),
@@ -205,25 +193,10 @@ _COMPONENT_MAX_TRIANGLES = 2 ** 25
 
 
 def _mesh_device(mesh, device):
-    lib = _lib.load_library()
-    if not torch.cuda.is_available():
-        raise RuntimeError("image_to_pointcloud_b200 needs a CUDA device (no CPU fallback exists)")
+    lib, dev = _lib.load_library(), device_for(mesh.vertices, device)
     if len(mesh.triangles) > _COMPONENT_MAX_TRIANGLES or len(mesh.vertices) > 2 ** 31:
         raise ValueError("meshes of at most 2^25 triangles and 2^31 vertices are supported")
-    if isinstance(mesh.vertices, torch.Tensor):
-        return lib, mesh.vertices.device
-    return lib, torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-
-
-def _raise_component_errors(err: int, where: str) -> None:
-    if err & ~3:
-        raise RuntimeError(f"{where}: a device loop exhausted its bound (error word {err})")
-    if err:
-        raise ValueError("; ".join(msg for bit, msg in _COMPONENT_ERRORS if err & bit))
-
-
-def _ptr(t):
-    return t.data_ptr() if t is not None and t.numel() > 0 else None
+    return lib, dev
 
 
 def cluster_connected_triangles(mesh: TriangleMesh, *, device=None, return_device: bool = False):
@@ -235,25 +208,19 @@ def cluster_connected_triangles(mesh: TriangleMesh, *, device=None, return_devic
     lib, dev = _mesh_device(mesh, device)
     nv, nt = len(mesh.vertices), len(mesh.triangles)
     with torch.cuda.device(dev):
-        xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
-        tri = _device_array(mesh.triangles, torch.int32, 3, dev)
-        nb = C.c_size_t(0)
-        check(lib.d2pc_mesh_components_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_components_scratch_bytes")
-        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+        xyz = upload(mesh.vertices, torch.float32, 3, dev)
+        tri = upload(mesh.triangles, torch.int32, 3, dev)
+        buf = scratch(lib.d2pc_mesh_components_scratch_bytes, nv, nt, dev=dev)
         labels = torch.empty(nt, dtype=torch.int32, device=dev)
         n = torch.empty(nt, dtype=torch.int64, device=dev)
         area = torch.empty(nt, dtype=torch.float64, device=dev)
         words = torch.zeros(2, dtype=torch.int32, device=dev)   # K, error
-        check(lib.d2pc_mesh_components_enqueue(_ptr(xyz), nv, _ptr(tri), nt, scratch.data_ptr(), scratch.numel(),
-                                               _ptr(labels), _ptr(n), _ptr(area), words.data_ptr(),
-                                               words.data_ptr() + 4, _stream(dev)),
+        check(lib.d2pc_mesh_components_enqueue(ptr(xyz), nv, ptr(tri), nt, buf.data_ptr(), buf.numel(), ptr(labels),
+                                               ptr(n), ptr(area), words.data_ptr(), words.data_ptr() + 4, stream(dev)),
               "d2pc_mesh_components_enqueue")
         k, err = (int(v) for v in words.cpu())
-        _raise_component_errors(err, "cluster_connected_triangles")
-        out = (labels, n[:k], area[:k])
-        if return_device:
-            return out
-        return tuple(t.cpu().numpy() for t in out)
+        raise_errors(err, _COMPONENT_ERRORS, "cluster_connected_triangles")
+        return to_host((labels, n[:k], area[:k]), return_device)
 
 
 def remove_triangles_by_mask(mesh: TriangleMesh, mask, *, remove_unreferenced: bool = True, device=None,
@@ -274,35 +241,10 @@ def remove_triangles_by_mask(mesh: TriangleMesh, mask, *, remove_unreferenced: b
 
 
 def _filter(lib, dev, mesh, keep, remove_unreferenced, return_device):
-    nv, nt = len(mesh.vertices), len(mesh.triangles)
-    xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
-    rgb = _device_array(mesh.colors, torch.float32, 3, dev)
-    tri = _device_array(mesh.triangles, torch.int32, 3, dev)
-    rows = _device_array(mesh.vertex_rows, torch.int64, 0, dev)
-    nrm = None if mesh.vertex_normals is None else _device_array(mesh.vertex_normals, torch.float64, 3, dev)
-    if len(rgb) != nv or len(rows) != nv or (nrm is not None and len(nrm) != nv):
-        raise ValueError("colors, vertex_rows and vertex_normals must have one row per vertex")
-    nb = C.c_size_t(0)
-    check(lib.d2pc_mesh_filter_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_filter_scratch_bytes")
-    scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
-    oxyz = torch.empty((nv, 3), dtype=torch.float32, device=dev)
-    orgb = torch.empty((nv, 3), dtype=torch.float32, device=dev)
-    orow = torch.empty(nv, dtype=torch.int64, device=dev)
-    onrm = torch.empty((nv, 3), dtype=torch.float64, device=dev) if nrm is not None else None
-    otri = torch.empty((nt, 3), dtype=torch.int32, device=dev)
-    words = torch.zeros(3, dtype=torch.int32, device=dev)   # vertices, triangles, error
-    flags = (_lib.MESH_REMOVE_UNREFERENCED if remove_unreferenced else 0) | (_lib.MESH_NORMALS if nrm is not None else 0)
-    check(lib.d2pc_mesh_filter_enqueue(_ptr(xyz), _ptr(rgb), _ptr(nrm), _ptr(rows), nv, _ptr(tri), nt, _ptr(keep),
-                                       flags, scratch.data_ptr(), scratch.numel(), _ptr(oxyz), _ptr(orgb), _ptr(onrm),
-                                       _ptr(orow), words.data_ptr(), _ptr(otri), words.data_ptr() + 4,
-                                       words.data_ptr() + 8, _stream(dev)),
-          "d2pc_mesh_filter_enqueue")
-    kv, kt, err = (int(v) for v in words.cpu())
-    _raise_component_errors(err, "remove_triangles_by_mask")
-    out = TriangleMesh(oxyz[:kv], orgb[:kv], otri[:kt], onrm[:kv] if onrm is not None else None, orow[:kv])
-    if return_device:
-        return out
-    return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in out))
+    flags = (_lib.MESH_REMOVE_UNREFERENCED if remove_unreferenced else 0) | \
+        (_lib.MESH_NORMALS if mesh.vertex_normals is not None else 0)
+    return _reduce_mesh(lib.d2pc_mesh_filter_scratch_bytes, lib.d2pc_mesh_filter_enqueue, mesh, ptr(keep), flags,
+                        _COMPONENT_ERRORS, "remove_triangles_by_mask", dev, return_device)
 
 
 def check_min_triangles(min_triangles) -> int:
@@ -366,12 +308,6 @@ def _finite(name, x) -> float:
     return x
 
 
-def _host_or_device(out, return_device):
-    if return_device:
-        return out
-    return TriangleMesh(*(t.cpu().numpy() if t is not None else None for t in out))
-
-
 def _smooth(mesh, method, iterations, lambda_filter, mu, scope, device, return_device):
     n = check_iterations(iterations)
     lam, mu = _finite("lambda_filter", lambda_filter), _finite("mu", mu)
@@ -380,34 +316,17 @@ def _smooth(mesh, method, iterations, lambda_filter, mu, scope, device, return_d
     lib, dev = _mesh_device(mesh, device)
     nv, nt = len(mesh.vertices), len(mesh.triangles)
     with torch.cuda.device(dev):
-        xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
-        rgb = _device_array(mesh.colors, torch.float32, 3, dev)
-        tri = _device_array(mesh.triangles, torch.int32, 3, dev)
-        rows = _device_array(mesh.vertex_rows, torch.int64, 0, dev)
-        nrm = None if mesh.vertex_normals is None else _device_array(mesh.vertex_normals, torch.float64, 3, dev)
-        if len(rgb) != nv or len(rows) != nv or (nrm is not None and len(nrm) != nv):
-            raise ValueError("colors, vertex_rows and vertex_normals must have one row per vertex")
-        nb = C.c_size_t(0)
-        check(lib.d2pc_mesh_smooth_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_smooth_scratch_bytes")
-        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+        xyz, rgb, tri, rows, nrm = _mesh_inputs(mesh, dev)
+        buf = scratch(lib.d2pc_mesh_smooth_scratch_bytes, nv, nt, dev=dev)
         oxyz = torch.empty((nv, 3), dtype=torch.float32, device=dev)
         orgb = torch.empty((nv, 3), dtype=torch.float32, device=dev)
         onrm = torch.empty((nv, 3), dtype=torch.float64, device=dev) if nrm is not None else None
         err = torch.zeros(1, dtype=torch.int32, device=dev)
-        check(lib.d2pc_mesh_smooth_enqueue(_ptr(xyz), _ptr(rgb), _ptr(nrm), nv, _ptr(tri), nt, method, n, lam, mu,
-                                           SMOOTH_SCOPES[scope], scratch.data_ptr(), scratch.numel(), _ptr(oxyz),
-                                           _ptr(orgb), _ptr(onrm), err.data_ptr(), _stream(dev)),
-              "d2pc_mesh_smooth_enqueue")
-        e = int(err.cpu())
-        _raise_smooth_errors(e, "mesh smoothing")
-        return _host_or_device(TriangleMesh(oxyz, orgb, tri, onrm, rows), return_device)
-
-
-def _raise_smooth_errors(err: int, where: str) -> None:
-    if err & ~3:
-        raise RuntimeError(f"{where}: a device loop exhausted its bound (error word {err})")
-    if err:
-        raise ValueError("; ".join(msg for bit, msg in _SMOOTH_ERRORS if err & bit))
+        check(lib.d2pc_mesh_smooth_enqueue(ptr(xyz), ptr(rgb), ptr(nrm), nv, ptr(tri), nt, method, n, lam, mu,
+                                           SMOOTH_SCOPES[scope], buf.data_ptr(), buf.numel(), ptr(oxyz), ptr(orgb),
+                                           ptr(onrm), err.data_ptr(), stream(dev)), "d2pc_mesh_smooth_enqueue")
+        raise_errors(int(err.cpu()), _SMOOTH_ERRORS, "mesh smoothing")
+        return to_host(TriangleMesh(oxyz, orgb, tri, onrm, rows), return_device)
 
 
 def filter_smooth_simple(mesh: TriangleMesh, number_of_iterations: int = 1, *, scope: str = "all", device=None,
@@ -446,22 +365,14 @@ def compute_vertex_normals(mesh: TriangleMesh, *, device=None, return_device: bo
     lib, dev = _mesh_device(mesh, device)
     nv, nt = len(mesh.vertices), len(mesh.triangles)
     with torch.cuda.device(dev):
-        xyz = _device_array(mesh.vertices, torch.float32, 3, dev)
-        rgb = _device_array(mesh.colors, torch.float32, 3, dev)
-        tri = _device_array(mesh.triangles, torch.int32, 3, dev)
-        rows = _device_array(mesh.vertex_rows, torch.int64, 0, dev)
-        if len(rgb) != nv or len(rows) != nv:
-            raise ValueError("colors and vertex_rows must have one row per vertex")
-        nb = C.c_size_t(0)
-        check(lib.d2pc_mesh_vertex_normals_scratch_bytes(nv, nt, C.byref(nb)), "d2pc_mesh_vertex_normals_scratch_bytes")
-        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
+        xyz, rgb, tri, rows, _ = _mesh_inputs(mesh, dev, normals=False)
+        buf = scratch(lib.d2pc_mesh_vertex_normals_scratch_bytes, nv, nt, dev=dev)
         onrm = torch.empty((nv, 3), dtype=torch.float64, device=dev)
         err = torch.zeros(1, dtype=torch.int32, device=dev)
-        check(lib.d2pc_mesh_vertex_normals_enqueue(_ptr(xyz), nv, _ptr(tri), nt, scratch.data_ptr(), scratch.numel(),
-                                                   _ptr(onrm), err.data_ptr(), _stream(dev)),
-              "d2pc_mesh_vertex_normals_enqueue")
-        _raise_smooth_errors(int(err.cpu()), "compute_vertex_normals")
-        return _host_or_device(TriangleMesh(xyz, rgb, tri, onrm, rows), return_device)
+        check(lib.d2pc_mesh_vertex_normals_enqueue(ptr(xyz), nv, ptr(tri), nt, buf.data_ptr(), buf.numel(), ptr(onrm),
+                                                   err.data_ptr(), stream(dev)), "d2pc_mesh_vertex_normals_enqueue")
+        raise_errors(int(err.cpu()), _SMOOTH_ERRORS, "compute_vertex_normals")
+        return to_host(TriangleMesh(xyz, rgb, tri, onrm, rows), return_device)
 
 
 def lattice_shape(img_h: int, img_w: int, density: str):
@@ -501,20 +412,9 @@ def depth_to_mesh(image: np.ndarray, depth: np.ndarray, density: str = "medium",
     _cos2(max_angle), _max_edge(max_edge)   # argument errors before any device work
     if min_component_triangles is not None:
         check_min_triangles(min_component_triangles)
+    dev, xyz, rgb, _ = _lattice_emit(image, depth, density, invert, depth_scale, smooth, smooth_ksize, fov, device)
     img_h, img_w = image.shape[:2]
-    dep_h, dep_w = depth.shape[:2]
-    check_depth_dtype(depth, int(img_h), int(img_w))
-    img_c = _image_channels(image)
-    eng = _engine_for(int(img_h), int(img_w), img_c, int(dep_h), int(dep_w), device)
-    dev = eng.device
-    cfg = eng.make_config(density=density, invert=invert, depth_scale=float(depth_scale), fov=fov)
-    with eng._staging["lock"], torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev)
-        d = torch.from_numpy(np.ascontiguousarray(depth, dtype=np.float32).reshape(1, dep_h, dep_w)).to(dev)
-        im = torch.from_numpy(np.ascontiguousarray(image).reshape(1, img_h, img_w, -1)).to(dev) if img_c >= 3 else None
-        res = eng.process(cfg, d, im, stream=stream, smooth_ksize=(smooth_ksize if smooth else None))
-        n = eng.points_per_frame(cfg)
-        xyz, rgb = res.xyz[0, :n], res.rgb[0, :n]
+    with torch.cuda.device(dev):
         keep = None
         if z_range is not None:   # z32 >= f32(z_min) and z32 <= f32(z_max)
             z = xyz[:, 2]

@@ -16,8 +16,8 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._device import device_rows, row_bounds, scratch, stream, to_host
 from ._lib import check
-from .writers import _device_rows, _stream
 
 MAX_KNN = 64
 
@@ -43,7 +43,7 @@ def estimate_normals(points, *, knn: int = 30, radius=None, orient_towards=(0.0,
         if cam.shape != (3,) or not np.isfinite(cam).all():
             raise ValueError("orient_towards must be three finite numbers or None")
     lib = _lib.load_library()
-    xyz, _, count, n = _device_rows(points, None, device)
+    xyz, _, count, n = device_rows(points, None, device)
     dev = xyz.device
     with torch.cuda.device(dev):
         normals = torch.empty((n, 3), dtype=torch.float64, device=dev)
@@ -51,22 +51,14 @@ def estimate_normals(points, *, knn: int = 30, radius=None, orient_towards=(0.0,
         if n > 0:
             if not bool(torch.isfinite(xyz).all()):
                 raise ValueError("estimate_normals: non-finite coordinates")
-            nb = C.c_size_t(0)
-            check(lib.d2pc_normals_scratch_bytes(n, C.byref(nb)), "d2pc_normals_scratch_bytes")
-            scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
-            keys = torch.empty(6, dtype=torch.int32, device=dev)
-            bounds = torch.empty(6, dtype=torch.float32, device=dev)
-            s = _stream(dev)
-            check(lib.d2pc_rows_bounds_enqueue(xyz.data_ptr(), count.data_ptr(), n, keys.data_ptr(), bounds.data_ptr(), s),
-                  "d2pc_rows_bounds_enqueue")
+            buf = scratch(lib.d2pc_normals_scratch_bytes, n, dev=dev)
+            bounds = row_bounds(xyz, count, n, dev)
             cam_c = (C.c_double * 3)(*cam) if cam is not None else None
             check(lib.d2pc_normals_enqueue(xyz.data_ptr(), count.data_ptr(), n, bounds.data_ptr(), knn, r,
-                                           1 if cam is not None else 0, cam_c, scratch.data_ptr(), scratch.numel(),
-                                           normals.data_ptr(), cov.data_ptr() if cov is not None else None, s),
-                  "d2pc_normals_enqueue")
+                                           1 if cam is not None else 0, cam_c, buf.data_ptr(), buf.numel(),
+                                           normals.data_ptr(), cov.data_ptr() if cov is not None else None,
+                                           stream(dev)), "d2pc_normals_enqueue")
         if cov is not None:
             cov = cov[:, [0, 1, 2, 1, 3, 4, 2, 4, 5]].reshape(n, 3, 3)
-        if not return_device:
-            normals = normals.cpu().numpy()
-            cov = cov.cpu().numpy() if cov is not None else None
+        normals, cov = to_host((normals, cov), return_device)
         return (normals, cov) if return_covariances else normals

@@ -18,16 +18,15 @@ Each step is the same kernel sequence the individual drop-ins use, so the result
 """
 from __future__ import annotations
 
-import ctypes as C
 from pathlib import Path
 from typing import Optional
 
 import numpy as np
 import torch
 
-from . import _lib, cluster, writers
-from ._lib import check
-from .api import _engine_for, _image_channels, _to_host, bounds_dict, check_depth_dtype
+from . import cluster, writers
+from ._device import pinned, row_bounds
+from .api import _lattice_emit, bounds_dict
 from .engine import DENSITY_STEP
 from .mesh import (_cos2, _max_edge, _small_components, check_iterations, check_min_triangles, check_voxel_size,
                    compute_vertex_normals, filter_smooth_taubin, grid_mesh, lattice_shape, simplify_mesh)
@@ -85,21 +84,9 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
         cluster_eps = cluster.check_eps(cluster_eps, "cluster_eps")
         cluster_min_points = cluster.check_min_points(cluster_min_points, "cluster_min_points")
         cluster_min_size = cluster.check_min_size(cluster_min_size, "cluster_min_size")
-    lib = _lib.load_library()
+    dev, xyz, rgb, n = _lattice_emit(image, depth, density, invert, depth_scale, smooth, smooth_ksize, fov, device)
     img_h, img_w = image.shape[:2]
-    dep_h, dep_w = depth.shape[:2]
-    check_depth_dtype(depth, int(img_h), int(img_w))
-    img_c = _image_channels(image)
-    eng = _engine_for(int(img_h), int(img_w), img_c, int(dep_h), int(dep_w), device)
-    dev = eng.device
-    cfg = eng.make_config(density=density, invert=invert, depth_scale=float(depth_scale), fov=fov)
     with torch.cuda.device(dev):
-        stream = torch.cuda.current_stream(dev)
-        d = torch.from_numpy(np.ascontiguousarray(depth, dtype=np.float32).reshape(1, dep_h, dep_w)).to(dev)
-        im = torch.from_numpy(np.ascontiguousarray(image).reshape(1, img_h, img_w, -1)).to(dev) if img_c >= 3 else None
-        res = eng.process(cfg, d, im, stream=stream, smooth_ksize=(smooth_ksize if smooth else None))
-        n = int(res.count.cpu()[0])
-        xyz, rgb = res.xyz[0, :n], res.rgb[0, :n]
         lat_xyz, lat_rgb, kept = xyz, rgb, None   # the emit rows are the unmasked lattice
         if refine and n > 0:
             xyz, rgb, kept, _ = statistical_outlier_removal(xyz, rgb, nb_neighbors, std_ratio, return_device=True)
@@ -113,18 +100,14 @@ def point_cloud_stage(image: np.ndarray, depth: np.ndarray, *, density: str = "m
         out["point_count"] = m
         nrm = estimate_normals(xyz, knn=normals_knn, return_device=True) if normals else None
         if return_arrays:
-            out["points"], out["colors"] = _to_host(xyz), _to_host(rgb)   # pinned D2H at PCIe speed
+            out["points"], out["colors"] = pinned(xyz), pinned(rgb)
             if normals:
                 out["normals"] = nrm.cpu().numpy()
         pp, pc = writers.preview_lists(xyz, rgb, max_preview)
         out["preview_points"], out["preview_colors"] = pp, pc
         if m > 0:
             cnt = torch.tensor([m], dtype=torch.int32, device=dev)
-            keys = torch.empty(6, dtype=torch.int32, device=dev)
-            b6 = torch.empty(6, dtype=torch.float32, device=dev)
-            check(lib.d2pc_rows_bounds_enqueue(xyz.data_ptr(), cnt.data_ptr(), m, keys.data_ptr(), b6.data_ptr(),
-                                               stream.cuda_stream), "d2pc_rows_bounds_enqueue")
-            out["bounds"] = bounds_dict(b6.cpu().numpy())
+            out["bounds"] = bounds_dict(row_bounds(xyz, cnt, m, dev).cpu().numpy())
         fmt = (output_format or "").lower()
         if fmt:
             if fmt == "ply":

@@ -8,15 +8,14 @@ Same signature, return value and error convention as the reference: ``(points_f,
 """
 from __future__ import annotations
 
-import ctypes as C
 import logging
 
 import numpy as np
 import torch
 
 from . import _lib
+from ._device import device_rows, row_bounds, scratch, stream, to_host
 from ._lib import check
-from .writers import _device_rows, _stream
 
 logger = logging.getLogger(__name__)
 
@@ -26,33 +25,25 @@ def statistical_outlier_removal(points, colors=None, nb_neighbors: int = 20, std
     """-> (points_f, colors_f or None, kept_index, stats) with stats = dict(cloud_mean, std_dev, threshold)."""
     lib = _lib.load_library()
     has_colors = colors is not None and len(colors) == len(points)
-    xyz, rgb, count, n = _device_rows(points, colors if has_colors else None, device)
+    xyz, rgb, count, n = device_rows(points, colors if has_colors else None, device)
     dev = xyz.device
     with torch.cuda.device(dev):
-        nb = C.c_size_t(0)
-        check(lib.d2pc_sor_scratch_bytes(n, C.byref(nb)), "d2pc_sor_scratch_bytes")
-        scratch = torch.empty(int(nb.value), dtype=torch.uint8, device=dev)
-        keys = torch.empty(6, dtype=torch.int32, device=dev)
-        bounds = torch.empty(6, dtype=torch.float32, device=dev)
-        s = _stream(dev)
-        check(lib.d2pc_rows_bounds_enqueue(xyz.data_ptr(), count.data_ptr(), n, keys.data_ptr(), bounds.data_ptr(), s),
-              "d2pc_rows_bounds_enqueue")
+        buf = scratch(lib.d2pc_sor_scratch_bytes, n, dev=dev)
+        bounds = row_bounds(xyz, count, n, dev)
         oxyz = torch.empty_like(xyz)
         orgb = torch.empty_like(rgb) if has_colors else None
         oidx = torch.empty(n, dtype=torch.int32, device=dev)
         ocnt = torch.zeros(1, dtype=torch.int32, device=dev)
         stats = torch.zeros(4, dtype=torch.float64, device=dev)
         check(lib.d2pc_sor_enqueue(xyz.data_ptr(), rgb.data_ptr() if has_colors else None, count.data_ptr(), n,
-                                   bounds.data_ptr(), int(nb_neighbors), float(std_ratio), scratch.data_ptr(),
-                                   scratch.numel(), oxyz.data_ptr(), orgb.data_ptr() if has_colors else None,
-                                   oidx.data_ptr(), ocnt.data_ptr(), stats.data_ptr(), s), "d2pc_sor_enqueue")
+                                   bounds.data_ptr(), int(nb_neighbors), float(std_ratio), buf.data_ptr(), buf.numel(),
+                                   oxyz.data_ptr(), orgb.data_ptr() if has_colors else None, oidx.data_ptr(),
+                                   ocnt.data_ptr(), stats.data_ptr(), stream(dev)), "d2pc_sor_enqueue")
         m = int(ocnt.cpu()[0])
         st = stats.cpu().numpy()
         info = {"cloud_mean": float(st[0]), "std_dev": float(st[1]), "threshold": float(st[2])}
-        if return_device:
-            return oxyz[:m], (orgb[:m] if has_colors else None), oidx[:m], info
-        return (oxyz[:m].cpu().numpy(), orgb[:m].cpu().numpy() if has_colors else None,
-                oidx[:m].cpu().numpy().astype(np.int64), info)
+        pts, cols, idx = to_host((oxyz[:m], orgb[:m] if has_colors else None, oidx[:m]), return_device)
+        return pts, cols, (idx if return_device else idx.astype(np.int64)), info
 
 
 def refine_point_cloud(points, colors, nb_neighbors: int = 20, std_ratio: float = 2.0) -> tuple:

@@ -19,7 +19,6 @@ neither library is installed in the build container, so those two are "parity un
 """
 from __future__ import annotations
 
-import ctypes as C
 import datetime
 import logging
 import struct
@@ -30,6 +29,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._device import device_for, device_rows, pinned, row_bounds, scratch, stream, upload
 from ._lib import check
 
 logger = logging.getLogger(__name__)
@@ -41,41 +41,12 @@ PLY_FACE_RECORD_BYTES = 13
 MAX_PREVIEW = 20000  # app.py:496
 
 
-def _device_rows(points, colors, device=None):
-    """-> (xyz [n,3] f32 cuda, rgb [n,3] f32 cuda, count int32 [1] cuda, n)"""
-    if not torch.cuda.is_available():
-        raise RuntimeError("image_to_pointcloud_b200 needs a CUDA device (no CPU fallback exists)")
-    if isinstance(points, torch.Tensor):
-        xyz = points
-        dev = xyz.device
-    else:
-        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-        xyz = torch.from_numpy(np.ascontiguousarray(points, dtype=np.float32)).to(dev)
-    n = int(xyz.shape[0])
-    if colors is None or len(colors) != n:
-        # the reference's writers fall back to grey when there are no colours (app.py:371-374, 386)
-        rgb = torch.full((n, 3), 128.0, dtype=torch.float32, device=dev)
-    elif isinstance(colors, torch.Tensor):
-        rgb = colors.to(dev)
-    else:
-        rgb = torch.from_numpy(np.ascontiguousarray(colors, dtype=np.float32)).to(dev)
-    if xyz.dtype != torch.float32 or rgb.dtype != torch.float32 or xyz.dim() != 2 or xyz.shape[1] != 3:
-        raise ValueError("points / colors must be float32 [N, 3]")
-    xyz, rgb = xyz.contiguous(), rgb.contiguous()
-    count = torch.tensor([n], dtype=torch.int32, device=dev)
-    return xyz, rgb, count, n
-
-
-def _stream(dev) -> int:
-    return torch.cuda.current_stream(dev).cuda_stream
-
-
 # ---- preview (app.py:495-506) ----------------------------------------------------------------
 def preview_rows(points, colors, max_preview: int = MAX_PREVIEW, device=None) -> Tuple[np.ndarray, np.ndarray]:
     """points[::stride], colors[::stride] with the reference's stride rule, gathered on the device so
     only the preview rows cross PCIe."""
     lib = _lib.load_library()
-    xyz, rgb, count, n = _device_rows(points, colors, device)
+    xyz, rgb, count, n = device_rows(points, colors, device)
     cap = max(1, min(n, 2 * max_preview + 1))
     with torch.cuda.device(xyz.device):
         oxyz = torch.empty((cap, 3), dtype=torch.float32, device=xyz.device)
@@ -84,7 +55,7 @@ def preview_rows(points, colors, max_preview: int = MAX_PREVIEW, device=None) ->
         if n > 0:
             check(lib.d2pc_preview_rows_enqueue(xyz.data_ptr(), rgb.data_ptr(), count.data_ptr(), int(max_preview),
                                                 oxyz.data_ptr(), orgb.data_ptr(), cap, ocnt.data_ptr(),
-                                                _stream(xyz.device)), "d2pc_preview_rows_enqueue")
+                                                stream(xyz.device)), "d2pc_preview_rows_enqueue")
         m = int(ocnt.cpu()[0])
         return oxyz[:m].cpu().numpy(), orgb[:m].cpu().numpy()
 
@@ -98,30 +69,26 @@ def preview_lists(points, colors, max_preview: int = MAX_PREVIEW, device=None):
 # ---- XYZ ASCII (app.py:379-389) ---------------------------------------------------------------
 def xyz_text(points, colors, device=None) -> bytes:
     lib = _lib.load_library()
-    xyz, rgb, count, n = _device_rows(points, colors, device)
+    xyz, rgb, count, n = device_rows(points, colors, device)
     if n == 0:
         return b""
     dev = xyz.device
     with torch.cuda.device(dev):
-        nbytes = C.c_size_t(0)
-        check(lib.d2pc_xyz_text_scratch_bytes(n, C.byref(nbytes)), "d2pc_xyz_text_scratch_bytes")
-        scratch = torch.empty(int(nbytes.value), dtype=torch.uint8, device=dev)
+        buf = scratch(lib.d2pc_xyz_text_scratch_bytes, n, dev=dev)
         total = torch.zeros(1, dtype=torch.int64, device=dev)
         err = torch.zeros(1, dtype=torch.int32, device=dev)
         check(lib.d2pc_xyz_text_measure_enqueue(xyz.data_ptr(), rgb.data_ptr(), count.data_ptr(), n,
-                                                scratch.data_ptr(), scratch.numel(), total.data_ptr(),
-                                                err.data_ptr(), _stream(dev)), "d2pc_xyz_text_measure_enqueue")
+                                                buf.data_ptr(), buf.numel(), total.data_ptr(),
+                                                err.data_ptr(), stream(dev)), "d2pc_xyz_text_measure_enqueue")
         if int(err.cpu()[0]) != 0:
             # the reference raises here as well (int(nan) / int(inf)); huge magnitudes are not supported
             raise ValueError("cannot format the point cloud as XYZ text (non-finite colour or |coordinate| >= 2^44)")
         size = int(total.cpu()[0])
         text = torch.empty(size + 16, dtype=torch.uint8, device=dev)
         check(lib.d2pc_xyz_text_write_enqueue(xyz.data_ptr(), rgb.data_ptr(), count.data_ptr(), n,
-                                              scratch.data_ptr(), scratch.numel(), total.data_ptr(), err.data_ptr(),
-                                              text.data_ptr(), size, _stream(dev)), "d2pc_xyz_text_write_enqueue")
-        host = torch.empty(size, dtype=torch.uint8, pin_memory=True)
-        host.copy_(text[:size])
-        return host.numpy().tobytes()
+                                              buf.data_ptr(), buf.numel(), total.data_ptr(), err.data_ptr(),
+                                              text.data_ptr(), size, stream(dev)), "d2pc_xyz_text_write_enqueue")
+        return pinned(text[:size]).tobytes()
 
 
 def save_xyz(points, colors, filename: str, device=None) -> str:
@@ -137,30 +104,26 @@ def save_xyz(points, colors, filename: str, device=None) -> str:
 def las_point_records(points, colors, scale: float = 0.01, offsets=None, device=None):
     """-> (records uint8 [n, 26], offsets [3] float, int_minmax int32 [6])."""
     lib = _lib.load_library()
-    xyz, rgb, count, n = _device_rows(points, colors, device)
+    xyz, rgb, count, n = device_rows(points, colors, device)
     if n == 0:
         raise ValueError("No points to write to LAS")
     dev = xyz.device
     with torch.cuda.device(dev):
-        bounds = torch.zeros(6, dtype=torch.float32, device=dev)
         if offsets is None:  # float(points[:, k].min()), app.py:352
-            keys = torch.empty(6, dtype=torch.int32, device=dev)
-            check(lib.d2pc_rows_bounds_enqueue(xyz.data_ptr(), count.data_ptr(), n, keys.data_ptr(), bounds.data_ptr(),
-                                               _stream(dev)), "d2pc_rows_bounds_enqueue")
+            bounds = row_bounds(xyz, count, n, dev)
             offsets = [float(v) for v in bounds[:3].cpu()]
         else:
+            bounds = torch.zeros(6, dtype=torch.float32, device=dev)
             bounds[:3] = torch.tensor([float(v) for v in offsets], dtype=torch.float32)
         rec = torch.empty(n * LAS_RECORD_BYTES + 16, dtype=torch.uint8, device=dev)
         mm = torch.zeros(6, dtype=torch.int32, device=dev)
         err = torch.zeros(1, dtype=torch.int32, device=dev)
         check(lib.d2pc_las_records_enqueue(xyz.data_ptr(), rgb.data_ptr(), count.data_ptr(), n, bounds.data_ptr(),
-                                           float(scale), rec.data_ptr(), mm.data_ptr(), err.data_ptr(), _stream(dev)),
+                                           float(scale), rec.data_ptr(), mm.data_ptr(), err.data_ptr(), stream(dev)),
               "d2pc_las_records_enqueue")
         if int(err.cpu()[0]) != 0:
             raise OverflowError("LAS: scaled coordinate does not fit int32 (laspy raises OverflowError here)")
-        host = torch.empty(n * LAS_RECORD_BYTES, dtype=torch.uint8, pin_memory=True)
-        host.copy_(rec[:n * LAS_RECORD_BYTES])
-        return host.numpy().reshape(n, LAS_RECORD_BYTES), list(offsets), mm.cpu().numpy()
+        return pinned(rec[:n * LAS_RECORD_BYTES]).reshape(n, LAS_RECORD_BYTES), list(offsets), mm.cpu().numpy()
 
 
 def las_header(n: int, scale: float, offsets, int_minmax) -> bytes:
@@ -201,21 +164,11 @@ PLY_NORMAL_HEADER = ("ply\nformat binary_little_endian 1.0\ncomment Created by O
                      "property uchar red\nproperty uchar green\nproperty uchar blue\nend_header\n")
 
 
-def _device_normals(normals, n: int, dev) -> torch.Tensor:
-    if isinstance(normals, torch.Tensor):
-        nrm = normals.to(dev)
-    else:
-        nrm = torch.from_numpy(np.ascontiguousarray(normals, dtype=np.float64)).to(dev)
-    if nrm.dtype != torch.float64 or tuple(nrm.shape) != (n, 3):
-        raise ValueError("normals must be float64 [N, 3] for N points")
-    return nrm.contiguous()
-
-
 def ply_vertex_records(points, colors, device=None, normals=None) -> np.ndarray:
     """-> uint8 [n, 27]: float64 x, y, z and uchar r, g, b per vertex; with ``normals`` (float64 [n, 3]) uint8
     [n, 51]: float64 x, y, z, nx, ny, nz and uchar r, g, b."""
     lib = _lib.load_library()
-    xyz, rgb, count, n = _device_rows(points, colors, device)
+    xyz, rgb, count, n = device_rows(points, colors, device)
     rb = PLY_RECORD_BYTES if normals is None else PLY_NORMAL_RECORD_BYTES
     if n == 0:
         return np.zeros((0, rb), np.uint8)
@@ -224,14 +177,15 @@ def ply_vertex_records(points, colors, device=None, normals=None) -> np.ndarray:
         rec = torch.empty(n * rb + 16, dtype=torch.uint8, device=dev)
         if normals is None:
             check(lib.d2pc_ply_records_enqueue(xyz.data_ptr(), rgb.data_ptr(), count.data_ptr(), n, rec.data_ptr(),
-                                               _stream(dev)), "d2pc_ply_records_enqueue")
+                                               stream(dev)), "d2pc_ply_records_enqueue")
         else:
-            nrm = _device_normals(normals, n, dev)
+            if tuple(np.shape(normals)) != (n, 3) or (isinstance(normals, torch.Tensor)
+                                                      and normals.dtype != torch.float64):
+                raise ValueError("normals must be float64 [N, 3] for N points")
+            nrm = upload(normals, torch.float64, 3, dev)
             check(lib.d2pc_ply_normal_records_enqueue(xyz.data_ptr(), nrm.data_ptr(), rgb.data_ptr(), count.data_ptr(),
-                                                      n, rec.data_ptr(), _stream(dev)), "d2pc_ply_normal_records_enqueue")
-        host = torch.empty(n * rb, dtype=torch.uint8, pin_memory=True)
-        host.copy_(rec[:n * rb])
-        return host.numpy().reshape(n, rb)
+                                                      n, rec.data_ptr(), stream(dev)), "d2pc_ply_normal_records_enqueue")
+        return pinned(rec[:n * rb]).reshape(n, rb)
 
 
 def save_ply(points, colors, filename: str, device=None, normals=None) -> str:
@@ -255,26 +209,20 @@ PLY_MESH_NORMAL_HEADER = PLY_NORMAL_HEADER.replace("end_header\n", PLY_FACE_ELEM
 def ply_face_records(triangles, device=None) -> np.ndarray:
     """-> uint8 [t, 13]: uchar 3 and the three vertex ids as uint32 per triangle (int32 [t, 3] in)."""
     lib = _lib.load_library()
-    if isinstance(triangles, torch.Tensor):
-        tri = triangles
-    else:
-        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-        tri = torch.from_numpy(np.ascontiguousarray(triangles, dtype=np.int32).reshape(-1, 3)).to(dev)
-    if tri.dtype != torch.int32 or tri.dim() != 2 or tri.shape[1] != 3:
+    if isinstance(triangles, torch.Tensor) and (triangles.dtype != torch.int32 or triangles.dim() != 2
+                                                or triangles.shape[1] != 3):
         raise ValueError("triangles must be int32 [T, 3]")
+    dev = device_for(triangles, device)
+    tri = upload(triangles, torch.int32, 3, dev)
     t = int(tri.shape[0])
     if t == 0:
         return np.zeros((0, PLY_FACE_RECORD_BYTES), np.uint8)
-    dev = tri.device
     with torch.cuda.device(dev):
-        tri = tri.contiguous()
         cnt = torch.tensor([t], dtype=torch.int32, device=dev)
         rec = torch.empty(t * PLY_FACE_RECORD_BYTES + 16, dtype=torch.uint8, device=dev)
-        check(lib.d2pc_ply_face_records_enqueue(tri.data_ptr(), cnt.data_ptr(), t, rec.data_ptr(), _stream(dev)),
+        check(lib.d2pc_ply_face_records_enqueue(tri.data_ptr(), cnt.data_ptr(), t, rec.data_ptr(), stream(dev)),
               "d2pc_ply_face_records_enqueue")
-        host = torch.empty(t * PLY_FACE_RECORD_BYTES, dtype=torch.uint8, pin_memory=True)
-        host.copy_(rec[:t * PLY_FACE_RECORD_BYTES])
-        return host.numpy().reshape(t, PLY_FACE_RECORD_BYTES)
+        return pinned(rec[:t * PLY_FACE_RECORD_BYTES]).reshape(t, PLY_FACE_RECORD_BYTES)
 
 
 def _mesh_ply_parts(mesh, device=None):

@@ -126,6 +126,24 @@ def test_drop_in_call_is_thread_safe():
     assert errors == []
 
 
+def test_stages_run_the_engine_under_its_lock(monkeypatch):
+    """point_cloud_stage and depth_to_mesh share the cached engine with the drop-in call, so they run it under the
+    same lock."""
+    import image_to_pointcloud_b200 as m
+    held = []
+    process = m.FrameEngine.process
+
+    def recording(self, *args, **kwargs):
+        held.append(self._staging["lock"].locked())
+        return process(self, *args, **kwargs)
+
+    monkeypatch.setattr(m.FrameEngine, "process", recording)
+    img, dep = cases.make_image(120, 160, 5), cases.make_depth(77, 103, 5, "uniform")
+    m.point_cloud_stage(img, dep, output_format=None, device="cuda:0")
+    m.depth_to_mesh(img, dep, device="cuda:0")
+    assert held == [True, True]
+
+
 def test_engine_on_a_device_that_is_not_current():
     """The library launches on the current device: FrameEngine makes its own device current around every call."""
     if torch.cuda.device_count() < 2:
